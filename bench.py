@@ -24,6 +24,8 @@ Timed region: barrier + synchronize on both sides, CUDA events on the launching 
                  stream), algorithmic bytes per launch from SURVEY.md 8(d) / DESIGN.md, peak from MEASURED_PEAKS.json.
 `cpu_baseline` : the reference's own cv2 call chain (aruco_detect.py:250-269,592-601) on the host cores, bounded sample,
                  1 thread and all threads, median and best per frame (BASELINE.md section 3).
+--dump-outputs DIR: what the last timed step returned to its caller (rank 0), one DIR/<name>.npy per array (dump_outputs).
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -63,6 +65,7 @@ KERNEL_NOTES = {
     "k_sparse_exact": "exact colour chain on the tiles the bounds pass could not rule out",
 }
 METRIC = "4K frames/s (undistort+ArUco detect+pose)"
+DUMP_BYTES = 64_000_000           # --dump-outputs: at most this much in all
 
 
 def load_camera():
@@ -343,6 +346,24 @@ def roofline_of(ktimes, frames_timed, alg_override=None):
             "kernel_note": KERNEL_NOTES.get(name)}
 
 
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: writes every array of `arrays` (name -> numpy array or torch tensor) as out_dir/<name>.npy.  Integers of
+    up to 16 bits and float32 are written as float32, everything else as float64 (exact either way).  An array larger than
+    its equal share of DUMP_BYTES is flattened and written at a fixed sample of its indices (seed 0, sorted), the same sample
+    in every run with the same arguments."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 128                  # 128: the .npy header
+    for name, a in arrays.items():
+        t = torch.from_numpy(np.ascontiguousarray(a)) if isinstance(a, np.ndarray) else a
+        dtype = torch.float32 if t.element_size() <= 2 or t.dtype == torch.float32 else torch.float64
+        cap = share // (4 if dtype == torch.float32 else 8)
+        if t.numel() > cap:
+            idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), cap))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.to(dtype).cpu().numpy())
+
+
 def collect_ktimes(engines):
     ktimes = {}
     for e in engines:
@@ -455,6 +476,8 @@ def run_sequence_workload(args, rank, world, local_rank):
     ms, wall_ms = c.timed(step, args.steps)
     launches = pipe.launches - l0
     sampler.stop_flag = True
+    if rank == 0 and args.dump_outputs:   # the CSV row fields (the CSV text is rendered from them)
+        dump_outputs(args.dump_outputs, {f: state["rows"][f] for f in state["rows"].dtype.names})
     # ---- the GPU pipeline alone on the same frames (no gather, no post-pass)
     step_pipeline(0)
     ms_pipe, _ = c.timed(step_pipeline, args.steps)
@@ -602,6 +625,8 @@ def run_preprocess_workload(args, rank, world, local_rank):
     ms, _ = c.timed(step, args.steps)
     launches = e.launches - l0
     sampler.stop_flag = True
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     e.timing(True)
     step(0)
     e.timing_collect(reset=True)
@@ -707,6 +732,8 @@ def run_dense_workload(args, rank, world, local_rank):
     ms, _ = c.timed(step, args.steps)
     launches = pipe.launches - l0
     sampler.stop_flag = True
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, state["det"])
     markers = int(state["det"]["n"].sum().item())
     for e in pipe.engines:
         e.timing(True)
@@ -774,7 +801,12 @@ def main():
     ap.add_argument("--ref-frames-per-step", type=int, default=2)
     ap.add_argument("--dense-batch", type=int, default=24)
     ap.add_argument("--classic-windows", type=int, nargs=3, default=[3, 23, 10], metavar=("MIN", "MAX", "STEP"))
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
