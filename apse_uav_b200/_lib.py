@@ -6,7 +6,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("APSE_LIB") or os.path.join(_HERE, "libapse_b200.so")   # APSE_LIB: development override (kernel variants)
+LIB_PATH = os.environ.get("APSE_LIB") or os.path.join(_HERE, "libapse_b200.so")   # APSE_LIB: another build of the library (make decprof)
 
 
 class ApseError(RuntimeError):

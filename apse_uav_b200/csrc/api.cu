@@ -273,13 +273,6 @@ int apse_fill_device_params(apse_ctx *ctx, DeviceParams *dp, int w, int h)
     return APSE_OK;
 }
 
-// development switch: APSE_DENSE=1 turns the sparse evaluation off everywhere (A/B runs of the two preprocess paths)
-static bool sparse_enabled()
-{
-    static const bool off = getenv("APSE_DENSE") != nullptr && getenv("APSE_DENSE")[0] == '1';
-    return !off;
-}
-
 // candidates (APRILTAG quad detector or the classic threshold / contour path) -> grouping + decoding -> SUBPIX
 static int apse_detect_impl(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, apse_detections *out, cudaStream_t st,
                             bool have_tile_minmax)
@@ -340,7 +333,7 @@ int apse_process_frames(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gray, int ba
     // K1 writes the 4x4-tile extrema of gray straight into the candidate stage's tile arrays.  A caller that does not ask for
     // the gray frames gets the sparse evaluation (identical detections; gray is computed only where the detector reads it).
     int rc = 1;
-    const bool sparse = want_sparse && sparse_enabled() && ctx->params.cornerRefinementMethod == 3 && !apse_quad_image_needed(ctx->params);
+    const bool sparse = want_sparse && ctx->params.cornerRefinementMethod == 3 && !apse_quad_image_needed(ctx->params);
     if (sparse) {
         rc = apse_preprocess_sparse(ctx, bgr, gray, ctx->tmm, 0, batch, ctx->params.aprilTagMinWhiteBlackDiff, st);
         if (rc < 0) return rc;
@@ -373,7 +366,7 @@ static int preprocess_tiles_impl(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gra
     int rc = 1;
     ctx->tiles_sparse[slot] = false;
     for (int k = 0; k < 2; k++) if (ctx->sparse_gray[k] == gray) ctx->sparse_gray[k] = nullptr;   // the buffer is rewritten now
-    if (want_sparse && sparse_enabled() && ctx->params.cornerRefinementMethod == 3 && !apse_quad_image_needed(ctx->params)) {
+    if (want_sparse && ctx->params.cornerRefinementMethod == 3 && !apse_quad_image_needed(ctx->params)) {
         rc = apse_preprocess_sparse(ctx, bgr, gray, ctx->tmm_buf[slot], slot, batch, ctx->params.aprilTagMinWhiteBlackDiff, (cudaStream_t)stream);
         if (rc < 0) return rc;
         if (rc == APSE_OK) { ctx->tiles_sparse[slot] = true; ctx->tiles_bgr[slot] = bgr; ctx->sparse_gray[slot] = gray; }

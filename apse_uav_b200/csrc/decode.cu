@@ -452,7 +452,7 @@ __device__ __forceinline__ int block_exclusive_scan(int v, int *s_scan)
 
 __global__ void __launch_bounds__(DEC_THREADS) k_decode(const uint8_t *__restrict__ gray, int w, int h, const float *__restrict__ quads,
                                                         const uint32_t *__restrict__ quad_order, int32_t *__restrict__ counters,
-                                                        DeviceParams P, const int32_t *__restrict__ dec_raw, int skip_decoded_parents,
+                                                        DeviceParams P, const int32_t *__restrict__ dec_raw,
                                                         unsigned char *__restrict__ big_scratch, size_t big_stride, int mid_tier, apse_detections out)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -708,9 +708,8 @@ __global__ void __launch_bounds__(DEC_THREADS) k_decode(const uint8_t *__restric
     // Acceptance, level by level from the innermost candidates outwards, as the dependency does it: a level's candidates are tried
     // (the group's main first, then its far-enough members); every accepted one marks its not yet seen ancestors, and each mark
     // counts as a processed candidate -- as does, again, the ancestor itself when its own level comes.  The loop ends when the count
-    // reaches the number of candidates, so outer candidates of a frame with nested markers may never be tried (and end up rejected);
-    // with skip_decoded_parents a marked ancestor is not tried at all.  Ancestors are strictly higher than their descendants, so
-    // the candidates of one level are independent of each other.
+    // reaches the number of candidates, so outer candidates of a frame with nested markers may never be tried (and end up rejected).
+    // Ancestors are strictly higher than their descendants, so the candidates of one level are independent of each other.
     const int max_depth = s_lvl[1];
     for (int dep = 0; dep <= max_depth; dep++) {
         if (s_lvl[0] >= ns) break;
@@ -719,7 +718,6 @@ __global__ void __launch_bounds__(DEC_THREADS) k_decode(const uint8_t *__restric
         for (int v = tid; v < ns; v += DEC_THREADS) {
             if (hgt[2 * v] != dep) continue;
             mine++;
-            if (skip_decoded_parents && hgt[2 * v + 1]) continue;
             const int head = A.sel[v];
             int use = -1;
             if (A.dec_valid[head]) use = head;
@@ -812,10 +810,7 @@ int apse_decode_candidates(apse_ctx *ctx, const uint8_t *gray, int w, int h, int
     int nb = dp.marker_size + 2 * dp.border_bits;
     if (nb * dp.cell_size > DEC_MAX_S || nb > 16 || dp.nbytes > 8)
         CTX_FAIL(ctx, APSE_ERR_UNSUPPORTED, "detect: canonical marker image %d px exceeds the %d px limit", nb * dp.cell_size, DEC_MAX_S);
-    // a quad that encloses an already decoded marker IS identified (cv2 4.13 on nested-marker frames, tests/test_gpu_detect.py);
-    // development switch APSE_SKIP_DECODED_PARENTS=1 restores the behaviour round 1 assumed
-    static const bool skip_env = getenv("APSE_SKIP_DECODED_PARENTS") != nullptr && getenv("APSE_SKIP_DECODED_PARENTS")[0] == '1';
-    int skip = skip_env ? 1 : 0;
+    // a quad that encloses an already decoded marker IS identified (cv2 4.13 on nested-marker frames, tests/test_gpu_detect.py)
     // hierarchy scratch of the quad fit is free at this point: [batch][APSE_MAX_QUADS] decode results
     int32_t *dec_raw = reinterpret_cast<int32_t *>(ctx->errs);
     const int cand_blocks = ctx->params.cornerRefinementMethod == 3 ? 64 : 512;   // CTAs per frame; a CTA without a candidate exits at once
@@ -828,7 +823,7 @@ int apse_decode_candidates(apse_ctx *ctx, const uint8_t *gray, int w, int h, int
     const int mid_tier = ctx->params.cornerRefinementMethod != 3 && ctx->decode_scratch ? 1 : 0;
     const size_t dec_smem = sizeof(DecodeSmem) + (mid_tier ? decode_arrays_small_bytes(DEC_MIDC) : decode_arrays_bytes(DEC_SMEMC));
     KLAUNCH(ctx, KID_DECODE, st, k_decode<<<batch, DEC_THREADS, dec_smem, st>>>(
-                gray, w, h, ctx->quads, ctx->quad_order, ctx->counters, dp, dec_raw, skip,
+                gray, w, h, ctx->quads, ctx->quad_order, ctx->counters, dp, dec_raw,
                 (unsigned char *)ctx->decode_scratch, decode_arrays_bytes(DEC_MAXC), mid_tier, *out));
     return APSE_OK;
 }

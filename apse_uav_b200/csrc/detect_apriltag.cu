@@ -544,107 +544,6 @@ __global__ void __launch_bounds__(CCL_THREADS) k_ccl_flatten(const uint8_t *__re
     }
 }
 
-// ---- connected components over the A-list (hot path) --------------------------------------------------------
-// The 32x16 CCL tiles above spend four pixels out of five on background.  Here a half-warp owns one 4x4 A-list tile:
-// the 16 ternary values become two 16-bit masks (one ballot), the union rule of the dependency becomes four edge masks
-// (E, S and -- white only -- SW, SE, each edge initiated by a pixel inside the dependency's loop ranges), and every lane
-// floods its own component with shifts and ANDs in registers; the lowest bit of the component is its tile-local root.
-// No shared memory, no atomics.  k_ccl_atile_merge then joins the components across tile borders in global memory.
-__global__ void __launch_bounds__(256) k_ccl_atile_local(const uint8_t *__restrict__ thresh, int w, int h, uint32_t *__restrict__ labels,
-                                                         const uint32_t *__restrict__ alist, const int *__restrict__ acount, int acap)
-{
-    const int n = min(*acount, acap);
-    const int lane = threadIdx.x & 31, sub = lane & 15, half = lane >> 4;
-    for (int it = (blockIdx.x * blockDim.x + threadIdx.x) >> 4; it - half < n; it += (gridDim.x * blockDim.x) >> 4) {
-        const bool live = it < n;
-        const uint32_t e = live ? alist[it] : 0u;
-        const int f = ATILE_F(e), x = ATILE_TX(e) * 4 + (sub & 3), y = ATILE_TY(e) * 4 + (sub >> 2);
-        const bool in = live && x < w && y < h;
-        const size_t base = (size_t)f * w * h;
-        const int v = in ? thresh[base + (size_t)y * w + x] : 127;
-        const bool src = v != 127 && x >= 1 && x <= w - 2 && y <= h - 2;
-        const uint32_t bw = __ballot_sync(0xffffffffu, v == 255), bb = __ballot_sync(0xffffffffu, v == 0), bs = __ballot_sync(0xffffffffu, src);
-        const uint32_t white = (bw >> (16 * half)) & 0xffffu, black = (bb >> (16 * half)) & 0xffffu, srcm = (bs >> (16 * half)) & 0xffffu;
-        const uint32_t eE = srcm & ((white & (white >> 1)) | (black & (black >> 1))) & 0x7777u;   // p -> p + 1, dx < 3
-        const uint32_t eS = srcm & ((white & (white >> 4)) | (black & (black >> 4)));              // p -> p + 4
-        const uint32_t eSW = srcm & (white & (white >> 3)) & 0x0eeeu;                              // p -> p + 3, dx > 0, dy < 3
-        const uint32_t eSE = srcm & (white & (white >> 5)) & 0x0777u;                              // p -> p + 5, dx < 3, dy < 3
-        uint32_t m = 1u << sub;
-        for (;;) {
-            const uint32_t g = ((m & eE) << 1) | ((m >> 1) & eE) | ((m & eS) << 4) | ((m >> 4) & eS) |
-                               ((m & eSW) << 3) | ((m >> 3) & eSW) | ((m & eSE) << 5) | ((m >> 5) & eSE);
-            const uint32_t m2 = m | g;
-            const bool grown = m2 != m;
-            m = m2;
-            if (!__any_sync(0xffffffffu, grown)) break;
-        }
-        if (in && v != 127) {
-            const int r = __ffs(m) - 1;
-            labels[base + (size_t)y * w + x] = (uint32_t)((ATILE_TY(e) * 4 + (r >> 2)) * w + ATILE_TX(e) * 4 + (r & 3));
-        }
-    }
-}
-
-// joins across A-list tile borders (global union-find on the tile-local roots).  Per tile 12 lanes: bottom row (S, SW, SE),
-// right column (E; SE for rows 0-2), left column rows 0-2 (SW); the other tile need not be listed itself -- a tile that is
-// not on the list holds 127.
-__global__ void __launch_bounds__(256) k_ccl_atile_merge(const uint8_t *__restrict__ thresh, int w, int h, uint32_t *__restrict__ labels,
-                                                         const uint32_t *__restrict__ alist, const int *__restrict__ acount, int acap)
-{
-    const int n = min(*acount, acap);
-    const int sub = threadIdx.x & 15;
-    for (int it = (blockIdx.x * blockDim.x + threadIdx.x) >> 4; it < n; it += (gridDim.x * blockDim.x) >> 4) {
-        if (sub >= 11) continue;
-        const uint32_t e = alist[it];
-        const int f = ATILE_F(e), x0 = ATILE_TX(e) * 4, y0 = ATILE_TY(e) * 4;
-        int x, y, kind;   // 0: bottom row (S, SW, SE leave the tile), 1: right column (E; SE for rows 0-2), 2: left column rows 0-2 (SW)
-        if (sub < 4) { kind = 0; x = x0 + sub; y = y0 + 3; }
-        else if (sub < 8) { kind = 1; x = x0 + 3; y = y0 + (sub - 4); }
-        else { kind = 2; x = x0; y = y0 + (sub - 8); }
-        if (x >= w || y >= h) continue;
-        if (x < 1 || x > w - 2 || y > h - 2) continue;   // not inside the dependency's loop ranges: initiates nothing
-        const uint8_t *t = thresh + (size_t)f * w * h;
-        uint32_t *L = labels + (size_t)f * w * h;
-        const uint32_t o = (uint32_t)(y * w + x);
-        const int v = t[o];
-        if (v == 127) continue;
-        // A union is skipped when two others imply it: pixels joined horizontally / vertically inside their own rows /
-        // columns carry the same component, so one union per pair of touching runs is enough.  srcx / srcy: the pixel
-        // at that column / row may initiate joins (the dependency's loop ranges); this pixel itself is a source.
-        auto srcx = [&](int xx) { return xx >= 1 && xx <= w - 2; };
-        const bool row1_src = y + 1 <= h - 2;            // pixels of row y + 1 may initiate joins
-        const bool s_same = t[o + w] == v;
-        if (kind == 0) {
-            const bool w_run = srcx(x - 1) && t[o - 1] == v;                          // (x-1,y) -E-> (x,y)
-            const bool e_run = srcx(x + 1) && t[o + 1] == v;                          // (x,y) -E-> (x+1,y), and (x+1,y) initiates its own S join
-            const bool sw_same = t[o + w - 1] == v, se_same = t[o + w + 1] == v;
-            const bool b_w_run = row1_src && srcx(x - 1) && sw_same && s_same;        // (x-1,y+1) -E-> (x,y+1)
-            const bool b_e_run = row1_src && s_same && se_same;                       // (x,y+1) -E-> (x+1,y+1)
-            if (s_same && !(w_run && b_w_run)) uf_union_gmem(L, o, o + w);
-            if (v == 255) {
-                if (sw_same && !(s_same && b_w_run) && !w_run) uf_union_gmem(L, o, o + w - 1);
-                if (se_same && !(s_same && b_e_run) && !e_run) uf_union_gmem(L, o, o + w + 1);
-            }
-        } else if (kind == 1) {
-            const bool e_same = t[o + 1] == v;
-            // E joins are never skipped: the skipped S joins rely on them (skipping both orientations would drop two edges
-            // of a 2x2 block that straddles a tile corner and leave only two of the three a spanning tree needs)
-            if (e_same) uf_union_gmem(L, o, o + 1);
-            if (v == 255 && sub < 7 && t[o + w + 1] == v) {
-                const bool via_e = e_same && srcx(x + 1);          // (x+1,y) -S-> (x+1,y+1)
-                const bool via_s = s_same && row1_src;             // (x,y+1) -E-> (x+1,y+1)
-                if (!via_e && !via_s) uf_union_gmem(L, o, o + w + 1);
-            }
-        } else {
-            if (v == 255 && t[o + w - 1] == v) {
-                const bool via_s = s_same && row1_src && srcx(x - 1);                  // (x-1,y+1) -E-> (x,y+1)
-                const bool via_w = srcx(x - 1) && t[o - 1] == v;                       // (x-1,y) -E-> (x,y), (x-1,y) -S-> (x-1,y+1)
-                if (!via_s && !via_w) uf_union_gmem(L, o, o + w - 1);
-            }
-        }
-    }
-}
-
 // ---------------------------------------------------------------------------------------------------------
 // K4: boundary points -> clusters
 __device__ __forceinline__ uint32_t hash64(unsigned long long k)
@@ -1363,11 +1262,10 @@ void apse_detect_free(apse_ctx *ctx)
     ctx->point_rank = nullptr;
 }
 
-// persistent grid of the work-list kernels (development knob APSE_CHAIN_GRID = CTAs per SM, default 2)
+// persistent grid of the work-list kernels: 2 CTAs per SM
 static int chain_grid(const apse_ctx *ctx)
 {
-    static const int per_sm = getenv("APSE_CHAIN_GRID") ? atoi(getenv("APSE_CHAIN_GRID")) : 2;
-    return ctx->sm_count * (per_sm > 0 ? per_sm : 1);
+    return ctx->sm_count * 2;
 }
 
 // runs K2..K5 for `batch` gray frames; leaves quads / counters in the context scratch
@@ -1420,27 +1318,18 @@ int apse_apriltag_quads(apse_ctx *ctx, const uint8_t *gray, int w, int h, int ba
                                                                                       ex->acap, ctx->thresh));
     }
     {
-        // development switch APSE_CCL_ATILES: components over the 4x4 A-list tiles (register flood + global border joins)
-        // instead of the 32x16 CCL tiles.  Validated (same results) but 1 % slower on sparse and 10 % slower on dense frames:
-        // the border joins of 4x4 tiles are four times as many global union-find operations.
-        static const bool ccl_atiles = getenv("APSE_CCL_ATILES") != nullptr;
-        if (flat_labels || !ccl_atiles) {
-            // 32x16 CCL tiles (shared-memory union-find); flat_labels (debug entry point): every pixel labelled with its
-            // component root.  Also the path of the classic detector (apse_ccl_binary).
-            int *n_active = ex->work_counter + 1;
-            KLAUNCH(ctx, KID_THRESHOLD, st, k_compact_tiles<<<div_up(batch * nct, 256), 256, 0, st>>>(ex->tile_active, batch * nct, nct, ex->tile_list, n_active));
-            const int block = CCL_THREADS;
-            const int grid = chain_grid(ctx) * 4;   // persistent: 16 CTAs of 128 threads per SM, tiles taken round-robin from the list
-            KLAUNCH(ctx, KID_CCL_LOCAL, st, k_ccl_local<<<grid, block, 0, st>>>(ctx->thresh, w, h, ctx->labels, ex->tile_list, n_active, ctw, 0));
-            KLAUNCH(ctx, KID_CCL_MERGE, st, k_ccl_merge<<<chain_grid(ctx) * 2, 256, 0, st>>>(ctx->thresh, w, h, ctx->labels, ex->tile_list, n_active, ctw, 0));
-            if (flat_labels)
-                KLAUNCH(ctx, KID_CCL_FLATTEN, st, k_ccl_flatten<<<grid, block, 0, st>>>(ctx->thresh, w, h, ctx->labels, ex->tile_list, n_active, ctw));
-        } else {
-            KLAUNCH(ctx, KID_CCL_LOCAL, st, k_ccl_atile_local<<<chain_grid(ctx), 256, 0, st>>>(ctx->thresh, w, h, ctx->labels, ex->alist[cur], acount, ex->acap));
-            static const int mg_per_sm = getenv("APSE_MERGE_GRID") ? atoi(getenv("APSE_MERGE_GRID")) : 16;
-            const int mg = ctx->sm_count * mg_per_sm;   // latency-bound root walks: many tiles in flight
-            KLAUNCH(ctx, KID_CCL_MERGE, st, k_ccl_atile_merge<<<mg, 256, 0, st>>>(ctx->thresh, w, h, ctx->labels, ex->alist[cur], acount, ex->acap));
-        }
+        // 32x16 CCL tiles (shared-memory union-find); flat_labels (debug entry point): every pixel labelled with its
+        // component root.  Also the path of the classic detector (apse_ccl_binary).  Components over the 4x4 A-list tiles
+        // (register flood + global border joins) gave the same results but ran 1 % slower on sparse and 10 % slower on
+        // dense frames: the border joins of 4x4 tiles are four times as many global union-find operations.
+        int *n_active = ex->work_counter + 1;
+        KLAUNCH(ctx, KID_THRESHOLD, st, k_compact_tiles<<<div_up(batch * nct, 256), 256, 0, st>>>(ex->tile_active, batch * nct, nct, ex->tile_list, n_active));
+        const int block = CCL_THREADS;
+        const int grid = chain_grid(ctx) * 4;   // persistent: 16 CTAs of 128 threads per SM, tiles taken round-robin from the list
+        KLAUNCH(ctx, KID_CCL_LOCAL, st, k_ccl_local<<<grid, block, 0, st>>>(ctx->thresh, w, h, ctx->labels, ex->tile_list, n_active, ctw, 0));
+        KLAUNCH(ctx, KID_CCL_MERGE, st, k_ccl_merge<<<chain_grid(ctx) * 2, 256, 0, st>>>(ctx->thresh, w, h, ctx->labels, ex->tile_list, n_active, ctw, 0));
+        if (flat_labels)
+            KLAUNCH(ctx, KID_CCL_FLATTEN, st, k_ccl_flatten<<<grid, block, 0, st>>>(ctx->thresh, w, h, ctx->labels, ex->tile_list, n_active, ctw));
         KLAUNCH(ctx, KID_EMIT, st, k_emit_scan<<<chain_grid(ctx), 256, 0, st>>>(ctx->thresh, w, h, ex->alist[cur], acount, ex->acap, ctx->points, ctx->counters));
         KLAUNCH(ctx, KID_EMIT, st, k_emit_insert<<<dim3(ctx->sm_count, min(batch, 8)), 256, 0, st>>>(w, h, ctx->labels, ctx->hash_keys, ctx->hash_count, ex->used_slots,
                                                                                          ctx->points, ctx->counters, batch));

@@ -600,8 +600,7 @@ int apse_preprocess_ex(apse_ctx *ctx, const uint8_t *bgr, uint8_t *bgr_out, uint
 {
     int w = ctx->w, h = ctx->h;
     PFN_tmapEncodeTiled enc = get_tmap_encoder();
-    static const bool force_generic = getenv("APSE_K1_GENERIC") != nullptr;   // development switch: generic kernel only
-    bool tma_ok = !force_generic && enc && (w % 4) == 0 && (h % 4) == 0 && ((w * 3) % 16) == 0 && w >= P2_TW && h >= P2_TH && ((uintptr_t)bgr % 16) == 0 && ctx->tables2;
+    bool tma_ok = enc && (w % 4) == 0 && (h % 4) == 0 && ((w * 3) % 16) == 0 && w >= P2_TW && h >= P2_TH && ((uintptr_t)bgr % 16) == 0 && ctx->tables2;
     CUtensorMap tmap;
     if (tma_ok) {
         // every global stride must be a multiple of 16 bytes (checked above); an encoder that still refuses the frame geometry
@@ -619,35 +618,26 @@ int apse_preprocess_ex(apse_ctx *ctx, const uint8_t *bgr, uint8_t *bgr_out, uint
         KLAUNCH(ctx, KID_PREPROCESS, st, k_preprocess_fused<<<grid, 256, 0, st>>>(bgr, bgr_out, gray, ctx->mapx, ctx->mapy, ctx->tables, w, h, batch, fpb));
         return 1;   // tile extrema not produced
     }
-    // registers per thread (development knob APSE_K1_NREG): at 64 the resident preprocess CTAs fill the register file and
-    // every CTA of the candidate / decode / pose chain on the other streams displaces one of them; 48 (no spills, 9 % fewer
-    // instructions than the 40-register build) = three 384-thread CTAs per SM with 10 K registers left for chain CTAs
-    static const int nreg = getenv("APSE_K1_NREG") ? atoi(getenv("APSE_K1_NREG")) : 48;
-    static const bool no_full = getenv("APSE_K1_NOFULL") != nullptr;   // development switch: no all-valid specialisation
+    // registers per thread at 4K: at 64 the resident preprocess CTAs fill the register file and every CTA of the
+    // candidate / decode / pose chain on the other streams displaces one of them; 48 (no spills, 9 % fewer instructions than
+    // the 40-register build) = three 384-thread CTAs per SM with 10 K registers left for chain CTAs
     if (!ctx->k1_attr_set) {
-        CUDA_TRY(ctx, cudaFuncSetAttribute(k_preprocess_tma<false, 64, 3840>, cudaFuncAttributeMaxDynamicSharedMemorySize, P2_SMEM_BYTES));
         CUDA_TRY(ctx, cudaFuncSetAttribute(k_preprocess_tma<false, 64, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, P2_SMEM_BYTES));
         CUDA_TRY(ctx, cudaFuncSetAttribute(k_preprocess_tma<true, 64, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, P2_SMEM_BYTES));
-        CUDA_TRY(ctx, cudaFuncSetAttribute(k_preprocess_tma<false, 40, 3840>, cudaFuncAttributeMaxDynamicSharedMemorySize, P2_SMEM_BYTES));
         CUDA_TRY(ctx, cudaFuncSetAttribute(k_preprocess_tma<false, 48, 3840>, cudaFuncAttributeMaxDynamicSharedMemorySize, P2_SMEM_BYTES));
         CUDA_TRY(ctx, cudaFuncSetAttribute(k_preprocess_tma<false, 48, 3840, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, P2_SMEM_BYTES));
         ctx->k1_attr_set = true;
     }
     // frames per CTA: the tap set-up (map reads, box reduction, table load) is amortised over up to 20 frames
-    static const int fpb_max = getenv("APSE_K1_FPB") ? atoi(getenv("APSE_K1_FPB")) : 20;   // development knob
-    const int nz = div_up(batch, fpb_max), fpb = div_up(batch, nz);
+    const int nz = div_up(batch, 20), fpb = div_up(batch, nz);
     dim3 grid(div_up(w, P2_TW), div_up(h, P2_TH), nz);
 #define K1T_ARGS tmap, bgr, bgr_out, gray, tmm, ctx->mapx, ctx->mapy, ctx->tables2, w, h, batch, fpb
     if (bgr_out)
         KLAUNCH(ctx, KID_PREPROCESS, st, k_preprocess_tma<true, 64, 0><<<grid, P2_CTA_THREADS, P2_SMEM_BYTES, st>>>(K1T_ARGS));
-    else if (w == 3840 && nreg == 40)
-        KLAUNCH(ctx, KID_PREPROCESS, st, k_preprocess_tma<false, 40, 3840><<<grid, P2_CTA_THREADS, P2_SMEM_BYTES, st>>>(K1T_ARGS));
-    else if (w == 3840 && nreg == 48 && h % P2_TH == 0 && !no_full)
+    else if (w == 3840 && h % P2_TH == 0)
         KLAUNCH(ctx, KID_PREPROCESS, st, k_preprocess_tma<false, 48, 3840, true><<<grid, P2_CTA_THREADS, P2_SMEM_BYTES, st>>>(K1T_ARGS));
-    else if (w == 3840 && nreg == 48)
-        KLAUNCH(ctx, KID_PREPROCESS, st, k_preprocess_tma<false, 48, 3840><<<grid, P2_CTA_THREADS, P2_SMEM_BYTES, st>>>(K1T_ARGS));
     else if (w == 3840)
-        KLAUNCH(ctx, KID_PREPROCESS, st, k_preprocess_tma<false, 64, 3840><<<grid, P2_CTA_THREADS, P2_SMEM_BYTES, st>>>(K1T_ARGS));
+        KLAUNCH(ctx, KID_PREPROCESS, st, k_preprocess_tma<false, 48, 3840><<<grid, P2_CTA_THREADS, P2_SMEM_BYTES, st>>>(K1T_ARGS));
     else
         KLAUNCH(ctx, KID_PREPROCESS, st, k_preprocess_tma<false, 64, 0><<<grid, P2_CTA_THREADS, P2_SMEM_BYTES, st>>>(K1T_ARGS));
 #undef K1T_ARGS
@@ -894,8 +884,7 @@ int apse_preprocess_sparse(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gray, uin
 {
     const int w = ctx->w, h = ctx->h;
     PFN_tmapEncodeTiled enc = get_tmap_encoder();
-    static const bool force_generic = getenv("APSE_K1_GENERIC") != nullptr;
-    const bool tma_ok = !force_generic && enc && (w % 4) == 0 && (h % 4) == 0 && ((w * 3) % 16) == 0 && w >= P2_TW && h >= P2_TH &&
+    const bool tma_ok = enc && (w % 4) == 0 && (h % 4) == 0 && ((w * 3) % 16) == 0 && w >= P2_TW && h >= P2_TH &&
                         ((uintptr_t)bgr % 16) == 0 && ctx->tables2 && ctx->btable && batch <= 64 && (w % 32) == 0 &&   // k_sparse_flags: 8 tiles per thread
                         ((uintptr_t)gray % 4) == 0;                                                                  // k_sparse_exact: 32-bit stores
     if (!tma_ok) return 1;
@@ -916,63 +905,42 @@ int apse_preprocess_sparse(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gray, uin
         CUDA_TRY(ctx, cudaMalloc((void **)&ctx->elist[slot], ntiles * sizeof(uint32_t)));
         CUDA_TRY(ctx, cudaMalloc((void **)&ctx->ecount[slot], sizeof(int)));
     }
-    // development knobs: registers per thread (40 leaves 15 K registers per SM to co-resident chain CTAs, 48 has no spill) and
-    // depth of the staging ring
-    static const int nreg = getenv("APSE_K1B_NREG") ? atoi(getenv("APSE_K1B_NREG")) : 40;
-    static const int nst = getenv("APSE_K1B_STAGES") ? atoi(getenv("APSE_K1B_STAGES")) : 3;
+    // 4K bounds pass: 40 registers per thread (leaves 15 K registers per SM to co-resident chain CTAs; 48 has no spill) and a
+    // staging ring of 3
     static bool attr_set[64] = {false};
     if (!attr_set[ctx->device & 63]) {
-#define K1B_ATTR(NR, NST)                                                                                                                     \
-        CUDA_TRY(ctx, cudaFuncSetAttribute(k_preprocess_tma<false, NR, 3840, true, 1, NST>, cudaFuncAttributeMaxDynamicSharedMemorySize, P2_SMEM_BYTES_N(1, NST)))
-        K1B_ATTR(48, 4); K1B_ATTR(48, 3); K1B_ATTR(48, 2); K1B_ATTR(40, 4); K1B_ATTR(40, 3); K1B_ATTR(40, 2);
-#undef K1B_ATTR
+        CUDA_TRY(ctx, cudaFuncSetAttribute(k_preprocess_tma<false, 40, 3840, true, 1, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, P2_SMEM_BYTES_N(1, 3)));
         CUDA_TRY(ctx, cudaFuncSetAttribute(k_preprocess_tma<false, 48, 0, false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, P2_SMEM_BYTES_M(1)));
         attr_set[ctx->device & 63] = true;
     }
-    static const int fpb_max = getenv("APSE_K1_FPB") ? atoi(getenv("APSE_K1_FPB")) : 20;
-    const int nz = div_up(batch, fpb_max), fpb = div_up(batch, nz);
+    const int nz = div_up(batch, 20), fpb = div_up(batch, nz);
     dim3 grid(div_up(w, P2_TW), div_up(h, P2_TH), nz);
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->ecount[slot], 0, sizeof(int), st));
 #define K1B_ARGS tmap, bgr, nullptr, nullptr, ctx->tbounds[slot], ctx->mapx, ctx->mapy, ctx->btable, w, h, batch, fpb
-#define K1B_GO(NR, NST) KLAUNCH(ctx, KID_PREPROCESS, st, k_preprocess_tma<false, NR, 3840, true, 1, NST><<<grid, P2_CTA_THREADS, P2_SMEM_BYTES_N(1, NST), st>>>(K1B_ARGS))
-    if (w == 3840 && h % P2_TH == 0) {
-        if (nreg == 40 && nst == 2) K1B_GO(40, 2);
-        else if (nreg == 40 && nst == 3) K1B_GO(40, 3);
-        else if (nreg == 40) K1B_GO(40, 4);
-        else if (nst == 2) K1B_GO(48, 2);
-        else if (nst == 3) K1B_GO(48, 3);
-        else K1B_GO(48, 4);
-    } else
+    if (w == 3840 && h % P2_TH == 0)
+        KLAUNCH(ctx, KID_PREPROCESS, st, k_preprocess_tma<false, 40, 3840, true, 1, 3><<<grid, P2_CTA_THREADS, P2_SMEM_BYTES_N(1, 3), st>>>(K1B_ARGS));
+    else
         KLAUNCH(ctx, KID_PREPROCESS, st, k_preprocess_tma<false, 48, 0, false, 1><<<grid, P2_CTA_THREADS, P2_SMEM_BYTES_M(1), st>>>(K1B_ARGS));
-#undef K1B_GO
 #undef K1B_ARGS
-    static const int exact_ctas = getenv("APSE_EXACT_CTAS") ? atoi(getenv("APSE_EXACT_CTAS")) : 6;   // CTAs per SM of k_sparse_exact
     // The two short kernels that follow gate the detector chain of this batch.  In a multi-stream pipeline they would share the
     // GPU with the bounds pass of the NEXT batch at its priority (0.2 - 0.6 ms instead of 0.04 + 0.10 ms, profiles/r02d_timeline.txt),
     // so they go to a high-priority stream of the context, fenced by two events: `st` sees them as if they had run on it.
-    // APSE_SPARSE_AUX=0: everything on `st`.
-    static const bool use_aux = !(getenv("APSE_SPARSE_AUX") && atoi(getenv("APSE_SPARSE_AUX")) == 0);
-    cudaStream_t sx = st;
-    if (use_aux) {
-        if (!ctx->aux_stream) {
-            int lo_prio = 0, hi_prio = 0;
-            CUDA_TRY(ctx, cudaDeviceGetStreamPriorityRange(&lo_prio, &hi_prio));
-            CUDA_TRY(ctx, cudaStreamCreateWithPriority(&ctx->aux_stream, cudaStreamNonBlocking, hi_prio));
-            CUDA_TRY(ctx, cudaEventCreateWithFlags(&ctx->aux_ev[0], cudaEventDisableTiming));
-            CUDA_TRY(ctx, cudaEventCreateWithFlags(&ctx->aux_ev[1], cudaEventDisableTiming));
-        }
-        sx = ctx->aux_stream;
-        CUDA_TRY(ctx, cudaEventRecord(ctx->aux_ev[0], st));
-        CUDA_TRY(ctx, cudaStreamWaitEvent(sx, ctx->aux_ev[0], 0));
+    if (!ctx->aux_stream) {
+        int lo_prio = 0, hi_prio = 0;
+        CUDA_TRY(ctx, cudaDeviceGetStreamPriorityRange(&lo_prio, &hi_prio));
+        CUDA_TRY(ctx, cudaStreamCreateWithPriority(&ctx->aux_stream, cudaStreamNonBlocking, hi_prio));
+        CUDA_TRY(ctx, cudaEventCreateWithFlags(&ctx->aux_ev[0], cudaEventDisableTiming));
+        CUDA_TRY(ctx, cudaEventCreateWithFlags(&ctx->aux_ev[1], cudaEventDisableTiming));
     }
+    cudaStream_t sx = ctx->aux_stream;
+    CUDA_TRY(ctx, cudaEventRecord(ctx->aux_ev[0], st));
+    CUDA_TRY(ctx, cudaStreamWaitEvent(sx, ctx->aux_ev[0], 0));
     KLAUNCH(ctx, KID_SPARSE_FLAGS, sx, k_sparse_flags<<<dim3(div_up(tw / 8, 128), div_up(th, SFL_ROWS), batch), 128, 0, sx>>>(
                 ctx->tbounds[slot], tw, th, min_wb_diff, tmm, ctx->eflag[slot], ctx->elist[slot], ctx->ecount[slot]));
-    KLAUNCH(ctx, KID_SPARSE_EXACT, sx, k_sparse_exact<<<ctx->sm_count * exact_ctas, 256, 0, sx>>>(bgr, ctx->mapx, ctx->mapy, ctx->tables2, w, h, ctx->elist[slot],
+    KLAUNCH(ctx, KID_SPARSE_EXACT, sx, k_sparse_exact<<<ctx->sm_count * 6, 256, 0, sx>>>(bgr, ctx->mapx, ctx->mapy, ctx->tables2, w, h, ctx->elist[slot],
                                                                                       ctx->ecount[slot], gray, tmm));
-    if (use_aux) {
-        CUDA_TRY(ctx, cudaEventRecord(ctx->aux_ev[1], sx));
-        CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->aux_ev[1], 0));
-    }
+    CUDA_TRY(ctx, cudaEventRecord(ctx->aux_ev[1], sx));
+    CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->aux_ev[1], 0));
     return APSE_OK;
 }
 

@@ -7,16 +7,10 @@ aruco_detect.py:598-782 runs afterwards on the host over the small per-frame res
 """
 from __future__ import annotations
 
-import os
-
 import numpy as np
 
 from .engine import Engine
 from ._lib import ApseError
-
-
-# development knob: APSE_SKIP_CHAIN=1 runs only the preprocess half in the multi-stream path (ceiling of that half; results are empty)
-_SKIP_CHAIN = os.environ.get("APSE_SKIP_CHAIN") == "1"
 
 
 class Pipeline:
@@ -46,18 +40,14 @@ class Pipeline:
         self.streams, self.pre_stream, self._gray, self._done = [], None, [], []
         self._ring, self._ring_size, self._ring_pos = {}, max(2, int(ring)), 0   # result buffers of run_batch(sync=False)
         if streams > 1:
-            # development knobs: stream priorities of the two halves (default: chain above preprocess)
-            pre_prio = int(os.environ.get("APSE_PRE_PRIO", "0"))
-            chain_prio = int(os.environ.get("APSE_CHAIN_PRIO", "-1"))
             # consecutive preprocess launches are independent (different frames, different contexts): rotating over
             # several streams lets the next launch fill the SMs while the last wave of the previous one drains, and lets the
             # short flag / exact kernels of one sub-batch run beside the bounds pass of the next (measured per 1800 frames:
             # 1 stream 52.7 ms, 2: 47.7, 3: 45.6, 4: 45.7, 6: 45.9)
-            n_pre = max(1, int(os.environ.get("APSE_PRE_STREAMS", "3")))
-            self.pre_streams = [torch.cuda.Stream(device=dev, priority=pre_prio) for _ in range(n_pre)]
+            self.pre_streams = [torch.cuda.Stream(device=dev, priority=0) for _ in range(3)]
             self.pre_stream = self.pre_streams[0]
             self._pre_pos = 0
-            self.streams = [torch.cuda.Stream(device=dev, priority=chain_prio) for _ in range(streams)]
+            self.streams = [torch.cuda.Stream(device=dev, priority=-1) for _ in range(streams)]
             # two gray buffers per engine (the library keeps two tile-extrema buffers to match): the preprocess of the next
             # use of engine s may run while the chain of the previous use still reads its gray / extrema; chains of one
             # engine are ordered by their stream, and a buffer is rewritten only after the chain two uses back has finished
@@ -167,8 +157,7 @@ class Pipeline:
                 sl = {k: v[lo:hi] for k, v in det.items()}
                 mls = ml[lo:hi] if isinstance(ml, torch.Tensor) else ml
                 with torch.cuda.stream(st):   # (a per-frame marker-length tensor is staged on the chain's stream)
-                    if not _SKIP_CHAIN:
-                        eng.detect_pose_frames(g, sl, mls, stream=st)
+                    eng.detect_pose_frames(g, sl, mls, stream=st)
                 self._done[s][par] = st.record_event()
                 done.append(self._done[s][par])
                 grays.append(g)

@@ -284,7 +284,7 @@ def _packed_fields(torch, cap, m):
     return fields, sizes_b, offs
 
 
-def run_sequence_streamed(pipe, frames, plan, rank=0, world=1, group=None, start_frame=1, as_rows=False, chunk_frames=240, post_thread=None):
+def run_sequence_streamed(pipe, frames, plan, rank=0, world=1, group=None, start_frame=1, as_rows=False, chunk_frames=240):
     """aruco_detect.py:571-810 for a sequence sharded by round_plan, with the post-pass streamed behind the pipeline.
     frames: this rank's parts of all rounds, concatenated ([n_local,H,W,3] uint8 CUDA tensor); plan: round_plan(...) of the whole
     sequence (the same on every rank).  Per round every rank enqueues its batch (no host synchronisation), packs the batch's
@@ -361,13 +361,9 @@ def run_sequence_streamed(pipe, frames, plan, rank=0, world=1, group=None, start
     # enqueueing thread each of them lets the pipeline's launch queue run dry: 57.4 against 54.2 ms per 1800 frames on one GPU).
     # The worker waits for the rounds in order and pushes them once chunk_frames frames have piled up; event / stream
     # synchronisation and the ctypes calls release the interpreter lock.  Waiting by polling with short sleeps was tried and is
-    # much worse (67 - 105 ms: every wake-up takes the lock away from the enqueueing thread).  post_thread=False /
-    # APSE_POST_THREAD=0: pushes between the enqueues of the calling thread.
-    import os
+    # much worse (67 - 105 ms: every wake-up takes the lock away from the enqueueing thread).
     import queue
     import threading
-    if post_thread is None:
-        post_thread = os.environ.get("APSE_POST_THREAD", "1") != "0"
     todo = queue.Queue()
     failure = []
 
@@ -386,7 +382,7 @@ def run_sequence_streamed(pipe, frames, plan, rank=0, world=1, group=None, start
             failure.append(exc)
 
     th = None
-    if rank == 0 and nr and post_thread:
+    if rank == 0 and nr:
         th = threading.Thread(target=worker, name="apse-postpass", daemon=True)
         th.start()
     try:
@@ -415,13 +411,6 @@ def run_sequence_streamed(pipe, frames, plan, rank=0, world=1, group=None, start
                     if th is not None:
                         todo.put(arrived[-1])
             lo += sz   # (after a failure of the worker the remaining rounds are still enqueued: the other ranks wait in their gathers)
-            if rank == 0 and th is None:
-                # no worker thread: completed rounds between the enqueues, once enough frames have piled up
-                ready = done_upto
-                while ready < len(arrived) and arrived[ready][1].query():
-                    ready += 1
-                if sum(hi_ - lo_ for rr in range(done_upto, ready) for lo_, hi_ in plan[rr]) >= chunk_frames:
-                    process(ready)
     except BaseException:
         if th is not None:
             todo.put((nr, None))
@@ -434,13 +423,6 @@ def run_sequence_streamed(pipe, frames, plan, rank=0, world=1, group=None, start
     if rank != 0:
         comm.synchronize()
         return None
-    if th is None:   # what is left: everything but the last round (its batch may still be running), then the last round
-        if nr - done_upto > 1:
-            arrived[nr - 2][1].synchronize()
-            process(nr - 1)
-        if nr:
-            arrived[nr - 1][1].synchronize()
-            process(nr)
     rows = seq.result()
     return rows if as_rows else sequence.rows_to_dicts(rows)
 

@@ -157,7 +157,7 @@ int apse_preprocess_tiles(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gray, int 
  * to become 127 in the detector's threshold image and are skipped; the others (+ a one-tile ring) and the samples of
  * candidate quads get the exact chain.  `gray` is a work buffer afterwards: complete only on the evaluated tiles and only
  * meaningful to the apse_detect_pose_frames call that follows on this context.  apse_process_frames(gray = NULL) takes this
- * path as well.  Falls back to apse_preprocess_tiles for frame geometries without a TMA path.  APSE_DENSE=1 disables it. */
+ * path as well.  Falls back to apse_preprocess_tiles for frame geometries without a TMA path. */
 int apse_preprocess_tiles_sparse(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gray, int batch, void *stream);
 int apse_detect_pose_frames(apse_ctx *ctx, const uint8_t *gray, int batch, apse_detections *out, const float *marker_len,
                             float marker_len_all, double *rvec, double *tvec, void *stream);
