@@ -9,6 +9,10 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("APSE_LIB") or os.path.join(_HERE, "libapse_b200.so")   # APSE_LIB: another build of the library (make decprof)
 
 
+# candidate quads per frame the library handles (APSE_MAX_QUADS, csrc/common.cuh): no frame can yield more markers or rejects
+MAX_QUADS = 4096
+
+
 class ApseError(RuntimeError):
     """Raised for every non-zero apse_status (mirrors cv2.error in the drop-in API)."""
 

@@ -7,6 +7,7 @@ import zlib
 import numpy as np
 
 from ._dict_data import DICTS as _DICTS
+from . import _lib
 from ._lib import ApseError
 from . import engine as _engine
 
@@ -111,7 +112,7 @@ def detectMarkers(image, dictionary, corners=None, ids=None, parameters=None, re
     raw, ms, mc = _dict_fields(dictionary)
     e.set_dictionary(raw, ms, mc)
     e.set_params(parameters if parameters is not None else DetectorParameters())
-    res = e.detect(img, max_markers=1024, want_rejected=True)
+    res = e.detect(img, max_markers=_lib.MAX_QUADS, want_rejected=True)   # room for every candidate: cv2 returns them all
     status = int(res["status"][0])
     if status != 0:
         raise ApseError(status, "detectMarkers: work-buffer capacity exceeded for this frame")

@@ -280,7 +280,10 @@ static int apse_detect_impl(apse_ctx *ctx, const uint8_t *gray, int w, int h, in
     DeviceParams dp;
     apse_fill_device_params(ctx, &dp, w, h);
     const int mode = ctx->params.cornerRefinementMethod;
-    int rc;
+    // both candidate paths can produce more than DEC_SMEMC candidates per frame (a 4K frame with a few hundred small markers
+    // does on the APRILTAG path): the decode stage then needs its global candidate arrays, whatever ran on the context before
+    int rc = apse_decode_big_scratch(ctx);
+    if (rc) return rc;
     if (mode == 3 && apse_quad_image_needed(ctx->params)) {
         // aprilTagQuadDecimate / aprilTagQuadSigma: quads are found on the shrunk / blurred image and scaled back; the tile
         // extrema of the full-size gray (if any) do not apply
@@ -294,8 +297,7 @@ static int apse_detect_impl(apse_ctx *ctx, const uint8_t *gray, int w, int h, in
     } else if (mode == 3) {
         rc = apse_apriltag_quads(ctx, gray, w, h, batch, dp, st, have_tile_minmax);
     } else {
-        rc = apse_decode_big_scratch(ctx);
-        if (!rc) rc = apse_classic_quads(ctx, gray, w, h, batch, st);
+        rc = apse_classic_quads(ctx, gray, w, h, batch, st);
     }
     if (rc) return rc;
     rc = apse_decode_candidates(ctx, gray, w, h, batch, dp, out, st);

@@ -738,7 +738,8 @@ __global__ void __launch_bounds__(AQ_WARPS * 32) k_approx_quads(ClassicArgs A)
     }
 }
 
-// rank of every quad of a frame in key order -> quad_order (consumed by the decode stage)
+// rank of every quad of a frame in key order -> quad_order (consumed by the decode stage).  Keys are unique within a frame
+// (classic: window and trigger pixel; APRILTAG: the cluster's component pair), so the ranks are a permutation.
 __global__ void k_rank_quads(const unsigned long long *__restrict__ keys, const int32_t *__restrict__ counters, int quad_cap,
                              uint32_t *__restrict__ quad_order)
 {
@@ -922,7 +923,7 @@ int apse_classic_quads(apse_ctx *ctx, const uint8_t *gray, int w, int h, int bat
         ClassicArgs A;
         A.pts = reinterpret_cast<uint32_t *>(ctx->sorted_pts); A.pts_cap = pts_cap;
         A.descs = reinterpret_cast<ContourDesc *>(ctx->clusters); A.desc_cap = desc_cap;
-        A.counters = ctx->counters; A.quads = ctx->quads; A.quad_keys = ctx->sort_keys; A.quad_cap = APSE_MAX_QUADS;
+        A.counters = ctx->counters; A.quads = ctx->quads; A.quad_keys = ctx->quad_keys; A.quad_cap = APSE_MAX_QUADS;
         A.refined = nullptr;
         if (p.cornerRefinementMethod == 2) {   // CORNER_REFINE_CONTOUR: the line fits need the contour, which only lives in this loop
             if (!ctx->quads_refined) CUDA_TRY(ctx, cudaMalloc((void **)&ctx->quads_refined, (size_t)ctx->max_batch * APSE_MAX_QUADS * 8 * sizeof(float)));
@@ -935,7 +936,14 @@ int apse_classic_quads(apse_ctx *ctx, const uint8_t *gray, int w, int h, int bat
         CUDA_TRY(ctx, cudaMemset2DAsync(ctx->counters, APSE_COUNTERS * sizeof(int32_t), 0, 2 * sizeof(int32_t), batch, st));
         CUDA_TRY(ctx, cudaMemset2DAsync(ctx->counters + 5, APSE_COUNTERS * sizeof(int32_t), 0, 2 * sizeof(int32_t), batch, st));   // [5] points, [6] long borders
     }
-    KLAUNCH(ctx, KID_APPROX, st, k_rank_quads<<<dim3(8, batch), 256, 0, st>>>(ctx->sort_keys, ctx->counters, APSE_MAX_QUADS, ctx->quad_order));
+    return apse_rank_quads(ctx, batch, st);
+}
+
+// both candidate paths: the decode stage breaks perimeter ties by this rank, so it has to be the dependency's candidate order
+int apse_rank_quads(apse_ctx *ctx, int batch, cudaStream_t st)
+{
+    const int kid = ctx->params.cornerRefinementMethod == 3 ? KID_FIT_QUADS : KID_APPROX;   // timed with the stage that made the quads
+    KLAUNCH(ctx, kid, st, k_rank_quads<<<dim3(8, batch), 256, 0, st>>>(ctx->quad_keys, ctx->counters, APSE_MAX_QUADS, ctx->quad_order));
     return APSE_OK;
 }
 

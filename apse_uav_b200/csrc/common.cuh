@@ -120,7 +120,8 @@ struct apse_ctx {
     ClusterDesc *clusters = nullptr;
     int32_t *counters = nullptr;      // per frame: {n_points, n_clusters_kept, n_quads, status, n_clusters_total, n_kept_points}
     float *quads = nullptr;           // [batch][APSE_MAX_QUADS][8]
-    uint32_t *quad_order = nullptr;   // cluster index of each quad (for deterministic ordering)
+    unsigned long long *quad_keys = nullptr;   // [batch][APSE_MAX_QUADS] candidate-order key of each quad (both candidate paths)
+    uint32_t *quad_order = nullptr;   // rank of each quad in the dependency's candidate order (apse_rank_quads)
     // decode scratch
     void *decode_scratch = nullptr;
     const uint8_t *tiles_gray[2] = {nullptr, nullptr};   // gray batch whose tile extrema are in tmm_buf[i] (apse_preprocess_tiles -> apse_detect_pose_frames)
@@ -228,6 +229,7 @@ int apse_apriltag_quads(apse_ctx *ctx, const uint8_t *gray, int w, int h, int ba
 int apse_decode_big_scratch(apse_ctx *ctx);
 int apse_adaptive_threshold_impl(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, int win, double c, uint8_t *out, cudaStream_t st);
 int apse_classic_quads(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, cudaStream_t st);
+int apse_rank_quads(apse_ctx *ctx, int batch, cudaStream_t st);   // ctx->quad_keys -> ctx->quad_order (keys unique per frame)
 int apse_contour_refine(apse_ctx *ctx, int batch, apse_detections *out, cudaStream_t st);
 int apse_corner_subpix(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, apse_detections *out, cudaStream_t st);
 int apse_decode_tap(apse_ctx *ctx, const uint8_t *gray, int w, int h, const float *corners, int n, const DeviceParams &dp, uint8_t *img_out,

@@ -24,7 +24,7 @@
 struct DecodeArrays {
     float (*c)[8];                        // candidate corners, sorted by perimeter (descending, stable)
     float *perim;
-    uint32_t *key;                        // ordering key (cluster index) / scratch
+    uint32_t *key;                        // ordering key (rank in the dependency's candidate order) / scratch
     uint32_t *close_bits;                 // [cap][cap / 32] words of scratch (centroid-test operands, bounding boxes; once a bit matrix)
     uint32_t *pairs;                      // [cap * 8] pairs (i << 16 | j) that pass the centroid pre-test, unordered
     float *cxy;                           // [cap][2] scratch: perimeters before the sort, group member lists, nesting heights
@@ -467,7 +467,7 @@ __global__ void __launch_bounds__(DEC_THREADS) k_decode(const uint8_t *__restric
     const int nq = min(cnt[2], DEC_MAXC);
     const float *q = quads + (size_t)f * APSE_MAX_QUADS * 8;
     const uint32_t *qo = quad_order + (size_t)f * APSE_MAX_QUADS;
-    if (nq > DEC_SMEMC && !big_scratch) {   // host passes the scratch whenever the path can produce this many quads
+    if (nq > DEC_SMEMC && !big_scratch) {   // apse_detect_impl always passes the scratch; without it such a frame is reported, not cut
         if (tid == 0) { out.n_markers[f] = 0; if (out.n_rejected) out.n_rejected[f] = 0; out.status[f] = APSE_ERR_CAPACITY; }
         return;
     }
@@ -794,7 +794,7 @@ int apse_decode_alloc(apse_ctx *ctx)
 }
 void apse_decode_free(apse_ctx *ctx) { cudaFree(ctx->decode_scratch); ctx->decode_scratch = nullptr; }
 
-// global candidate arrays for frames with more than DEC_SMEMC quads (classic path); allocated on first use
+// global candidate arrays for frames with more than DEC_SMEMC quads (either candidate path); allocated on first use
 int apse_decode_big_scratch(apse_ctx *ctx)
 {
     if (!ctx->decode_scratch) CUDA_TRY(ctx, cudaMalloc(&ctx->decode_scratch, decode_arrays_bytes(DEC_MAXC) * ctx->max_batch));

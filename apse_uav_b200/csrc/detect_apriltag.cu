@@ -834,7 +834,7 @@ struct FitArgs {
     double *lfps, *errs;
     int32_t *counters;
     float *quads;
-    uint32_t *quad_order;
+    unsigned long long *quad_keys;
     int *work_counter;
     int max_nmaxima;
     float critical_rad, max_line_fit_mse;
@@ -1184,7 +1184,8 @@ __global__ void __maxnreg__(40) k_fit_quads(FitArgs A)
                     float *q = A.quads + ((size_t)f * APSE_MAX_QUADS + qi) * 8;
                     const int order[4] = {3, 0, 1, 2};
                     for (int k = 0; k < 4; k++) { q[2 * k] = quad[order[k]][0]; q[2 * k + 1] = quad[order[k]][1]; }
-                    A.quad_order[(size_t)f * APSE_MAX_QUADS + qi] = (uint32_t)ci;
+                    // the dependency's candidate order is ascending cluster key (apse_rank_quads); qi follows thread scheduling
+                    A.quad_keys[(size_t)f * APSE_MAX_QUADS + qi] = ((unsigned long long)cd.key_hi << 32) | cd.key_lo;
                 } else {
                     atomicExch(&cnt[3], APSE_ERR_CAPACITY);
                 }
@@ -1228,6 +1229,7 @@ int apse_detect_alloc(apse_ctx *ctx)
     CUDA_TRY(ctx, cudaMalloc((void **)&ctx->counters, B * APSE_COUNTERS * sizeof(int32_t)));
     CUDA_TRY(ctx, cudaMalloc((void **)&ctx->quads, B * APSE_MAX_QUADS * 8 * sizeof(float)));
     CUDA_TRY(ctx, cudaMalloc((void **)&ctx->quad_order, B * APSE_MAX_QUADS * sizeof(uint32_t)));
+    CUDA_TRY(ctx, cudaMalloc((void **)&ctx->quad_keys, B * APSE_MAX_QUADS * sizeof(unsigned long long)));
     DetectExtra *ex = new DetectExtra();
     size_t nct = (size_t)div_up(ctx->max_w, CCL_TW) * div_up(ctx->max_h, CCL_TH);
     CUDA_TRY(ctx, cudaMalloc((void **)&ex->tile_active, B * nct));
@@ -1252,7 +1254,7 @@ void apse_detect_free(apse_ctx *ctx)
     cudaFree(ctx->thresh); cudaFree(ctx->tmm_buf[0]); cudaFree(ctx->tmm_buf[1]); cudaFree(ctx->labels); cudaFree(ctx->points);
     cudaFree(ctx->hash_keys); cudaFree(ctx->hash_count); cudaFree(ctx->hash_offset); cudaFree(ctx->sorted_pts);
     cudaFree(ctx->sort_keys); cudaFree(ctx->lfps); cudaFree(ctx->errs); cudaFree(ctx->clusters); cudaFree(ctx->counters);
-    cudaFree(ctx->quads); cudaFree(ctx->quad_order);
+    cudaFree(ctx->quads); cudaFree(ctx->quad_order); cudaFree(ctx->quad_keys);
     DetectExtra *ex = reinterpret_cast<DetectExtra *>(ctx->point_rank);
     if (ex) {
         cudaFree(ex->tile_active); cudaFree(ex->tile_list); cudaFree(ex->used_slots); cudaFree(ex->work_counter);
@@ -1340,10 +1342,10 @@ int apse_apriltag_quads(apse_ctx *ctx, const uint8_t *gray, int w, int h, int ba
     FitArgs A;
     A.gray = gray; A.w = w; A.h = h; A.batch = batch; A.clusters = ctx->clusters; A.sorted_pts = ctx->sorted_pts;
     A.sort_keys = ctx->sort_keys; A.lfps = ctx->lfps; A.errs = ctx->errs; A.counters = ctx->counters; A.quads = ctx->quads;
-    A.quad_order = ctx->quad_order; A.work_counter = ex->work_counter; A.max_nmaxima = dp.max_nmaxima;
+    A.quad_keys = ctx->quad_keys; A.work_counter = ex->work_counter; A.max_nmaxima = dp.max_nmaxima;
     A.critical_rad = dp.critical_rad; A.max_line_fit_mse = dp.max_line_fit_mse; A.max_dot = dp.max_dot;
     KLAUNCH(ctx, KID_FIT_QUADS, st, k_fit_quads<<<chain_grid(ctx) * 2, FQ_THREADS, 0, st>>>(A));   // one cluster per CTA at a time: dense frames have thousands
-    return APSE_OK;
+    return apse_rank_quads(ctx, batch, st);
 }
 
 // Components of a binary image for the classic path (classic.cu): foreground (255) 8-connected, background (0)

@@ -244,3 +244,55 @@ def make_inverted_frame(bytes_list, seed: int, width: int = 1920, height: int = 
         _paste_marker(frame, tile, quad, quiet_frac=8.0 / tile.shape[0])
     noise = rng.normal(0.0, noise_sigma, size=frame.shape).astype(np.float32)
     return np.clip(np.rint(frame.astype(np.float32) + noise), 0, 255).astype(np.uint8)
+
+
+def make_grid_frame(bytes_list, n: int, pitch: int = 64, side: int = 30, rotate: float = 0.0, seed: int = 0,
+                    width: int = 3840, height: int = 2160, noise_sigma: float = 2.0):
+    """Gray frame (uint8 HxW) with n markers on a grid (row by row, `pitch` px apart, ids 0..49 cycled) over a flat background of
+    128: many candidates per frame.  Every tile is rendered at its on-frame size (side px, quiet zone side // 6).  rotate = 0:
+    tiles pasted axis-aligned, every marker has the same perimeter; rotate > 0: each marker turned by a random angle of
+    rotate / 4 to rotate radians either way and shrunk by up to 15 % (distinct perimeters).  Raises if the grid holds fewer
+    than n markers."""
+    rng = np.random.default_rng(seed)
+    frame = np.full((height, width, 1), 128, np.uint8)
+    quiet = max(2, side // 6)
+    k = 0
+    for cy in range(pitch // 2 + 8, height - pitch // 2, pitch):
+        for cx in range(pitch // 2 + 8, width - pitch // 2, pitch):
+            if k >= n:
+                break
+            tile = render_marker(bytes_list, k % 50, side_px=side, quiet_px=quiet)
+            if rotate > 0:
+                # not near 0 (a marker turned by a few hundredths of a radian still fits to an axis-aligned quad), and a size
+                # that varies too (markers turned by +a and -a have the same perimeter)
+                a = rng.uniform(0.25, 1.0) * rotate * rng.choice((-1.0, 1.0))
+                c, s = np.cos(a), np.sin(a)
+                half = rng.uniform(0.85, 1.0) * side / 2
+                quad = np.float32([[-1, -1], [1, -1], [1, 1], [-1, 1]]) * half @ np.float32([[c, s], [-s, c]]) + np.float32([cx, cy])
+                _paste_marker(frame, tile, quad, quiet_frac=quiet / tile.shape[0])
+            else:
+                y0, x0 = cy - tile.shape[0] // 2, cx - tile.shape[1] // 2
+                frame[y0:y0 + tile.shape[0], x0:x0 + tile.shape[1], 0] = tile
+            k += 1
+    if k < n:
+        raise ValueError(f"a {width}x{height} grid of pitch {pitch} holds {k} markers, not {n}")
+    frame = frame[..., 0]
+    if noise_sigma > 0:
+        frame = np.clip(np.rint(frame + rng.normal(0, noise_sigma, frame.shape)), 0, 255).astype(np.uint8)
+    return frame
+
+
+def make_big_marker_frame(bytes_list, side: int, seed: int = 1, marker_id: int = 7, width: int = 3840, height: int = 2160,
+                          jitter: float = 0.03, noise_sigma: float = 3.0):
+    """BGR frame with ONE marker of about `side` px (rotated, corner jitter) in the middle of the textured background: boundary
+    clusters of thousands of points.  The tile is rendered sharp at its on-frame size (side // 6 * 6 px, quiet zone side // 12):
+    a small tile upscaled by the warp would have ramped edges, which neither cv2 nor the oracle detects at these sizes."""
+    rng = np.random.default_rng(seed)
+    frame = background(rng, width, height)
+    quiet = side // 12
+    tile = render_marker(bytes_list, marker_id, side_px=side // 6 * 6, quiet_px=quiet)
+    quad = _random_quad(rng, width / 2, height / 2, side, jitter)
+    _paste_marker(frame, tile, quad, quiet_frac=quiet / tile.shape[0])
+    if noise_sigma > 0:
+        frame = np.clip(np.rint(frame + rng.normal(0, noise_sigma, frame.shape)), 0, 255).astype(np.uint8)
+    return frame
