@@ -110,6 +110,7 @@ SIGNATURES = {
     "apse_sequence_csv": [_vp, _i, _i, _vp, _i64],
     "apse_debug_sparse": [_vp, _vp, _vp, _i, C.POINTER(C.c_int), _vp],
     "apse_debug_tile_bounds": [_vp, _vp, _i, _vp],
+    "apse_debug_tile_extrema": [_vp, _vp, _i, _vp],
     "apse_debug_decode": [_vp, _vp, _i, _i, _vp, _i, _vp, _vp, _vp, _vp],
     "apse_draw_overlay": [_vp, _vp, _i, _i, _i, _vp, _i, _vp],
     "apse_launch_count": [_vp],

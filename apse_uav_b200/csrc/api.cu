@@ -487,6 +487,18 @@ int apse_debug_tile_bounds(apse_ctx *ctx, uint16_t *bounds_dev, int batch, void 
     return APSE_OK;
 }
 
+int apse_debug_tile_extrema(apse_ctx *ctx, uint16_t *dst_dev, int batch, void *stream)
+{
+    if (!ctx || !dst_dev || batch <= 0 || batch > ctx->max_batch) CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "debug_tile_extrema: bad argument");
+    const int slot = ctx->tiles_slot ^ 1;   // the slot the last apse_preprocess_tiles[_sparse] call used
+    // tiles_gray[slot] is set only when that call produced extrema, and cleared by any call that drops them
+    if (!ctx->tiles_gray[slot]) CTX_FAIL(ctx, APSE_ERR_NOT_CONFIGURED, "debug_tile_extrema: the last preprocess_tiles batch left no tile extrema");
+    if (batch > ctx->tiles_batch[slot]) CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "debug_tile_extrema: batch %d exceeds the preprocessed batch %d", batch, ctx->tiles_batch[slot]);
+    CUDA_TRY(ctx, cudaMemcpyAsync(dst_dev, ctx->tmm_buf[slot], (size_t)batch * (ctx->w / 4) * (ctx->h / 4) * sizeof(uint16_t),
+                                  cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+    return APSE_OK;
+}
+
 int apse_debug_apriltag(apse_ctx *ctx, const uint8_t *gray, int w, int h, uint8_t *thresh, uint32_t *labels, float *quads,
                         int max_quads, int64_t *stats_host, void *stream)
 {

@@ -30,7 +30,7 @@ __global__ void k_tile_minmax(const uint8_t *__restrict__ gray, int w, int h, in
     if (tx >= tw || ty >= th) return;
     const uint8_t *g = gray + (size_t)f * w * h;
     unsigned mn = 255, mx = 0;
-    if ((w & 3) == 0) {
+    if ((w & 3) == 0 && (reinterpret_cast<uintptr_t>(gray) & 3) == 0) {   // 32-bit loads: every row 4-byte aligned
 #pragma unroll
         for (int dy = 0; dy < 4; dy++) {
             uint32_t v = __ldg(reinterpret_cast<const uint32_t *>(g + (size_t)(ty * 4 + dy) * w + tx * 4));
@@ -236,7 +236,7 @@ __global__ void __launch_bounds__(256) k_threshold_apply(const uint8_t *__restri
         if (tx >= tw || ty >= th) continue;   // partial edge tiles are written by k_threshold_edges
         const unsigned thr = alist_thr[i >> 2];
         const size_t p = (size_t)f * w * h + (size_t)(ty * 4 + dy) * w + tx * 4;
-        if ((w & 3) == 0) {
+        if ((w & 3) == 0 && (reinterpret_cast<uintptr_t>(gray) & 3) == 0) {   // out (thresh) is the context's own, aligned
             const uint32_t v = __ldg(reinterpret_cast<const uint32_t *>(gray + p));
             const uint32_t r = ((v & 255) > thr ? 0xffu : 0u) | (((v >> 8) & 255) > thr ? 0xff00u : 0u) |
                                (((v >> 16) & 255) > thr ? 0xff0000u : 0u) | ((v >> 24) > thr ? 0xff000000u : 0u);

@@ -196,7 +196,9 @@ __global__ void __launch_bounds__(256, 4) k_preprocess_fused(const uint8_t *__re
             g[k] = gray_px(o0[k], o1[k], o2[k]);
         }
         size_t o = (size_t)f * frame_px + (size_t)y * w + x0;
-        if (npx == K1_PX && (w & 3) == 0) {
+        // 32-bit stores need 4-byte aligned rows: the caller's buffers may start anywhere
+        if (npx == K1_PX && (w & 3) == 0 && (reinterpret_cast<uintptr_t>(gray) & 3) == 0 &&
+            (reinterpret_cast<uintptr_t>(bgr_out) & 3) == 0) {
             *reinterpret_cast<uint32_t *>(gray + o) = (uint32_t)g[0] | ((uint32_t)g[1] << 8) | ((uint32_t)g[2] << 16) | ((uint32_t)g[3] << 24);
             if (bgr_out) {
                 uint32_t *d = reinterpret_cast<uint32_t *>(bgr_out + o * 3);

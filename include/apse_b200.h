@@ -300,6 +300,12 @@ int apse_debug_sparse(apse_ctx *ctx, uint16_t *bound_table_host, uint8_t *eflag_
  * tile lies in [lo, hi]) */
 int apse_debug_tile_bounds(apse_ctx *ctx, uint16_t *bounds_dev, int batch, void *stream);
 
+/* test tap of the 4x4-tile extrema of gray that the last apse_preprocess_tiles[_sparse] call left for the detector (DEVICE,
+ * [batch][h/4][w/4], min | max << 8; after the sparse evaluation a tile that was not evaluated exactly holds (255, 0)).
+ * APSE_ERR_NOT_CONFIGURED when that call produced no extrema (the frame geometry took the generic kernel) or when another call
+ * on the context has dropped them since. */
+int apse_debug_tile_extrema(apse_ctx *ctx, uint16_t *dst_dev, int batch, void *stream);
+
 /* number of kernel launches issued through this context since creation (bench.py's gpu_launches) */
 int64_t apse_launch_count(apse_ctx *ctx);
 

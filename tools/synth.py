@@ -197,6 +197,43 @@ def make_nested_frame(bytes_list, seed: int, width: int = 1920, height: int = 10
     return frame, ids
 
 
+def make_edge_frame(bytes_list, seed: int, width: int, height: int, n_band: int = 6, noise_sigma: float = 3.0):
+    """BGR frame whose markers sit where the preprocess kernels have partial work: k_preprocess_tma covers the frame with CTAs of
+    64 x 24 output px, so a width or height that is not a multiple of those leaves a last CTA column or row with idle threads.
+    On the textured background, n_band rotated markers (side 34-52 px) straddle the left edge of the last CTA column
+    (x0 = width - width % 64, or width - 64) and n_band the top edge of the last CTA row (y0 likewise with 24), and three
+    markers are cut by the right and bottom frame edges (part of each in the last 8 px).  Positions are in the raw frame; the
+    undistortion moves them by a few pixels.  Frames narrower than 640 px get full-range colour noise over a colour gradient
+    instead (no marker fits)."""
+    rng = np.random.default_rng(seed)
+    if width < 640:
+        ramp = np.stack(np.broadcast_arrays((np.arange(width) * 255 // max(1, width - 1))[None, :],
+                                            (np.arange(height) * 255 // max(1, height - 1))[:, None],
+                                            ((np.arange(width)[None, :] + np.arange(height)[:, None]) * 4) % 256), -1)
+        noise = rng.integers(-60, 61, (height, width, 3))
+        return np.clip(ramp + noise, 0, 255).astype(np.uint8)
+    frame = background(rng, width, height)
+    x0 = width - (width % 64 or 64)
+    y0 = height - (height % 24 or 24)
+    ids = rng.choice(len(bytes_list), 2 * n_band + 3, replace=False)
+
+    def paste(mid, cx, cy, side):
+        tile = render_marker(bytes_list, int(mid))
+        _paste_marker(frame, tile, _random_quad(rng, cx, cy, side, 0.04), quiet_frac=8.0 / tile.shape[0])
+
+    for k in range(n_band):
+        side = float(rng.uniform(34, 52))
+        reach = side * 0.75 + 4                                   # half diagonal of the marker and its quiet zone
+        t = 0.12 + 0.6 * (k + rng.uniform(0.2, 0.8)) / n_band     # along the band, clear of the corner where the bands meet
+        paste(ids[2 * k], min(x0 + rng.uniform(-6, 14), width - reach), t * height, side)
+        paste(ids[2 * k + 1], t * width, min(y0 + rng.uniform(-6, 14), height - reach), side)
+    for j, (cx, cy) in enumerate(((width - 12, 0.8 * height), (0.85 * width, height - 12), (width - 10, height - 10))):
+        paste(ids[2 * n_band + j], cx, cy, float(rng.uniform(34, 52)))
+    if noise_sigma > 0:
+        frame = np.clip(np.rint(frame + rng.normal(0, noise_sigma, frame.shape)), 0, 255).astype(np.uint8)
+    return frame
+
+
 def make_sequence(bytes_list, base_seed: int, n_frames: int, width: int = 3840, height: int = 2160,
                   noise_sigma: float = 3.0, leds=None, events=None):
     """Sparse sequence (ids 1,2,3 = vehicles, 4 = host) with slow drift so that the track gating of
