@@ -6,7 +6,8 @@ vision-agh/apse_uav's aruco_detect.py.  Usage = an import swap at aruco_detect.p
 
 Hot functions (re-implemented as hand-written CUDA kernels behind libapse_b200.so, same signatures and
 return conventions as cv2): initUndistortRectifyMap (:568), remap (:252), cvtColor for COLOR_RGB2LAB /
-COLOR_LAB2RGB / COLOR_BGR2GRAY (:255,257,592), LUT (:256), undistort, projectPoints (:344,377,424,468),
+COLOR_LAB2RGB / COLOR_BGR2GRAY (:255,257,592) and for decoder output in YUV 4:2:0 (COLOR_YUV2BGR_NV12 / _NV21 / _I420 /
+_IYUV / _YV12), LUT (:256), undistort, projectPoints (:344,377,424,468),
 aruco.detectMarkers (:267), aruco.estimatePoseSingleMarkers (:601).  Everything else the script touches
 (VideoCapture, imread, imshow, putText, ...) is passed through to the installed cv2 when it is importable.
 
@@ -32,7 +33,9 @@ BORDER_CONSTANT = 0
 COLOR_BGR2GRAY, COLOR_RGB2GRAY = 6, 7
 COLOR_BGR2LAB, COLOR_RGB2LAB, COLOR_LAB2BGR, COLOR_LAB2RGB = 44, 45, 56, 57
 COLOR_BGR2Lab, COLOR_RGB2Lab, COLOR_Lab2BGR, COLOR_Lab2RGB = 44, 45, 56, 57
+COLOR_YUV2BGR_NV12, COLOR_YUV2BGR_NV21, COLOR_YUV2BGR_YV12, COLOR_YUV2BGR_I420, COLOR_YUV2BGR_IYUV = 91, 93, 99, 101, 101
 CV_32FC1, CV_16SC2 = 5, 11
+_YUV_CODES = {COLOR_YUV2BGR_NV12: "nv12", COLOR_YUV2BGR_NV21: "nv21", COLOR_YUV2BGR_YV12: "yv12", COLOR_YUV2BGR_I420: "i420"}
 
 
 def _is_torch(x):
@@ -72,10 +75,13 @@ def remap(src, map1, map2, interpolation, dst=None, borderMode=BORDER_CONSTANT, 
 
 
 def cvtColor(src, code, dst=None, dstCn=0):
-    """aruco_detect.py:255,257,592."""
+    """aruco_detect.py:255,257,592, and YUV 4:2:0 [H*3/2, W] -> BGR [H, W, 3] (COLOR_YUV2BGR_NV12 / _NV21 / _I420 / _YV12)."""
+    if code in _YUV_CODES:
+        e = default_engine(src.shape[-1], src.shape[-2] * 2 // 3)   # sized for the output frame, not the source's rows
+        return _out(e.cvt_yuv420(src, _YUV_CODES[code]), src)
     kinds = {COLOR_RGB2LAB: "rgb2lab", COLOR_LAB2RGB: "lab2rgb", COLOR_BGR2GRAY: "bgr2gray"}
     if code not in kinds:
-        raise ApseError(-5, f"cvtColor: conversion code {code} is not on the hot path (RGB2LAB, LAB2RGB, BGR2GRAY only)")
+        raise ApseError(-5, f"cvtColor: conversion code {code} is not on the hot path (RGB2LAB, LAB2RGB, BGR2GRAY, YUV2BGR_NV12 / NV21 / I420 / YV12 only)")
     e = default_engine(src.shape[1], src.shape[0])
     return _out(e.cvt(src, kinds[code]), src)
 

@@ -13,6 +13,10 @@ LIB_PATH = os.environ.get("APSE_LIB") or os.path.join(_HERE, "libapse_b200.so") 
 MAX_QUADS = 4096
 
 
+# apse_yuv_layout: YUV 4:2:0 layouts of apse_cvt_yuv420_bgr (cv2's single-array form [h*3/2][w])
+YUV_LAYOUTS = {"nv12": 0, "nv21": 1, "i420": 2, "yv12": 3}
+
+
 class ApseError(RuntimeError):
     """Raised for every non-zero apse_status (mirrors cv2.error in the drop-in API)."""
 
@@ -86,6 +90,7 @@ SIGNATURES = {
     "apse_cvt_lab2rgb": [_vp, _vp, _i64, _vp, _vp],
     "apse_cvt_bgr2gray": [_vp, _vp, _i64, _vp, _vp],
     "apse_lut": [_vp, _vp, _i64, _i, _vp, _vp, _i, _vp],
+    "apse_cvt_yuv420_bgr": [_vp, _vp, _i, _i, _i, _i, _vp, _vp],
     "apse_preprocess": [_vp, _vp, _vp, _vp, _i, _vp],
     "apse_detect": [_vp, _vp, _i, _i, _i, C.POINTER(Detections), _vp],
     "apse_pose": [_vp, _vp, _i, _vp, _f, _dp, _dp, _vp, _vp, _vp],

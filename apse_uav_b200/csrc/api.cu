@@ -98,7 +98,8 @@ static const char *KERNEL_NAMES[KID_COUNT] = {
     "k_build_undistort_map", "k_preprocess_fused", "k_remap", "k_cvt", "k_lut", "k_tile_minmax", "k_threshold",
     "k_ccl_local", "k_ccl_merge", "k_ccl_flatten", "k_emit_points", "k_cluster_scan", "k_scatter_points", "k_fit_quads",
     "k_decode", "k_pose", "k_project_points", "k_classic", "k_adaptive_threshold", "k_border_jobs", "k_trace_borders",
-    "k_approx_quads", "k_corner_subpix", "k_decode_bits", "k_sequence_jobs", "k_sparse_flags", "k_sparse_exact", "k_draw_overlay"};
+    "k_approx_quads", "k_corner_subpix", "k_decode_bits", "k_sequence_jobs", "k_sparse_flags", "k_sparse_exact", "k_draw_overlay",
+    "k_yuv420_to_bgr"};
 
 int apse_kernel_count(void) { return KID_COUNT; }
 const char *apse_kernel_name(int kid) { return kid >= 0 && kid < KID_COUNT ? KERNEL_NAMES[kid] : ""; }

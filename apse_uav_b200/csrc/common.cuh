@@ -68,7 +68,7 @@ enum KernelId {
     KID_BUILD_MAP = 0, KID_PREPROCESS, KID_REMAP, KID_CVT, KID_LUT, KID_TILE_MINMAX, KID_THRESHOLD, KID_CCL_LOCAL,
     KID_CCL_MERGE, KID_CCL_FLATTEN, KID_EMIT, KID_CLUSTER_SCAN, KID_SCATTER, KID_FIT_QUADS, KID_DECODE, KID_POSE,
     KID_PROJECT, KID_CLASSIC, KID_ADAPTIVE, KID_BORDER_JOBS, KID_TRACE, KID_APPROX, KID_SUBPIX, KID_DECODE_BITS, KID_SEQ_JOBS,
-    KID_SPARSE_FLAGS, KID_SPARSE_EXACT, KID_DRAW, KID_COUNT
+    KID_SPARSE_FLAGS, KID_SPARSE_EXACT, KID_DRAW, KID_YUV2BGR, KID_COUNT
 };
 #define APSE_EVENT_POOL 2048
 

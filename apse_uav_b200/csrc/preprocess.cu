@@ -2,6 +2,7 @@
 //   K0  build_undistort_map   aruco_detect.py:568  cv2.initUndistortRectifyMap
 //   K1  preprocess_fused      aruco_detect.py:250-259 + :592  remap + RGB2LAB + LUT(L) + LAB2RGB + BGR2GRAY
 //   stand-alone remap / cvtColor / LUT kernels for the drop-in cv2-shaped API
+//   k_yuv420_to_bgr: a video decoder's YUV 4:2:0 frames (NV12 / NV21 / I420 / YV12) -> BGR, cv2.cvtColor-exact
 // Integer pipeline, bit-exact with the dependency's 8-bit paths (SURVEY.md A.1, A.2).  HBM-bound by design:
 // one pass over the BGR frame (24.9 MB read) producing gray (8.3 MB) and optionally the corrected BGR frame.
 #include "common.cuh"
@@ -1081,6 +1082,146 @@ __global__ void k_lut(const uint8_t *__restrict__ src, int64_t n, int sstride, c
     __syncthreads();
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
         dst[i * dstride] = L[src[i * sstride]];
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// cv2.cvtColor(src, COLOR_YUV2BGR_{NV12,NV21,I420,YV12}): BT.601 limited range in 20-bit fixed point, no chroma
+// interpolation (the four pixels of a 2x2 block share one (U, V) pair).  Integer only, so bit-exact by construction.
+// One kernel for the four layouts: u / v point at the first chroma sample of frame 0, cstep is the element step of a chroma
+// row (2: interleaved, 1: planar), cstride its row stride; frames are fsz = w * h * 3 / 2 bytes apart.
+struct YuvTerms { int r, g, b; };
+
+__device__ __forceinline__ YuvTerms yuv_chroma(int U, int V)
+{
+    const int uu = U - 128, vv = V - 128, half = 1 << 19;
+    return {half + 1673527 * vv, half - 852492 * vv - 409993 * uu, half + 2116026 * uu};
+}
+
+__device__ __forceinline__ uint32_t yuv_px(int Y, const YuvTerms &c, int which)   // which: 0 B, 1 G, 2 R
+{
+    const int y = max(Y - 16, 0) * 1220542;
+    return (uint32_t)clip255((y + (which == 0 ? c.b : which == 1 ? c.g : c.r)) >> 20);
+}
+
+// scalar path: one thread per 2x2 block
+__global__ void __launch_bounds__(256) k_yuv420_to_bgr(const uint8_t *__restrict__ yp, const uint8_t *__restrict__ up,
+                                                       const uint8_t *__restrict__ vp, int cstep, int cstride, int w, int h,
+                                                       int batch, int64_t fsz, uint8_t *__restrict__ bgr)
+{
+    const int bw = w >> 1, nblk = bw * (h >> 1);
+    for (int f = blockIdx.y; f < batch; f += gridDim.y) {
+        for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < nblk; i += gridDim.x * blockDim.x) {
+            const int cy = i / bw, cx = i - cy * bw;
+            const int64_t co = f * fsz + (int64_t)cy * cstride + (int64_t)cx * cstep;
+            const YuvTerms c = yuv_chroma(up[co], vp[co]);
+#pragma unroll
+            for (int r = 0; r < 2; r++) {
+                const int64_t yo = (int64_t)f * fsz + (int64_t)(2 * cy + r) * w + 2 * cx;
+                uint8_t *d = bgr + ((int64_t)f * h * w + (int64_t)(2 * cy + r) * w + 2 * cx) * 3;
+#pragma unroll
+                for (int k = 0; k < 2; k++) {
+                    const int Y = yp[yo + k];
+                    d[3 * k] = (uint8_t)yuv_px(Y, c, 0);
+                    d[3 * k + 1] = (uint8_t)yuv_px(Y, c, 1);
+                    d[3 * k + 2] = (uint8_t)yuv_px(Y, c, 2);
+                }
+            }
+        }
+    }
+}
+
+// vector path (w % 16 == 0, 16-byte aligned source and destination): one thread = 2 rows x 16 columns.  Two 16-byte Y loads,
+// 16 bytes of interleaved chroma or 8 + 8 bytes from the two planes, 8 chroma triples, six 16-byte stores.
+template <int CSTEP>
+__global__ void __launch_bounds__(256) k_yuv420_to_bgr_v16(const uint8_t *__restrict__ yp, const uint8_t *__restrict__ up,
+                                                           const uint8_t *__restrict__ vp, int cstride, int w, int h, int batch,
+                                                           int64_t fsz, uint8_t *__restrict__ bgr)
+{
+    const int gw = w >> 4, ngrp = gw * (h >> 1);
+    for (int f = blockIdx.y; f < batch; f += gridDim.y) {
+        for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < ngrp; i += gridDim.x * blockDim.x) {
+            const int cy = i / gw, gx = i - cy * gw;
+            const int64_t co = f * fsz + (int64_t)cy * cstride + (int64_t)gx * 8 * CSTEP;
+            uint8_t U[8], V[8];
+            if (CSTEP == 2) {   // interleaved: up and vp are one byte apart, the lower of the two is 16-byte aligned
+                const uint4 q = __ldg(reinterpret_cast<const uint4 *>((up < vp ? up : vp) + co));
+                const uint32_t wd[4] = {q.x, q.y, q.z, q.w};
+                const int su = up < vp ? 0 : 8, sv = 8 - su;
+#pragma unroll
+                for (int k = 0; k < 8; k++) {
+                    U[k] = (uint8_t)(wd[k >> 1] >> ((k & 1) * 16 + su));
+                    V[k] = (uint8_t)(wd[k >> 1] >> ((k & 1) * 16 + sv));
+                }
+            } else {
+                const uint2 qu = __ldg(reinterpret_cast<const uint2 *>(up + co));
+                const uint2 qv = __ldg(reinterpret_cast<const uint2 *>(vp + co));
+#pragma unroll
+                for (int k = 0; k < 8; k++) {
+                    U[k] = (uint8_t)((k < 4 ? qu.x : qu.y) >> ((k & 3) * 8));
+                    V[k] = (uint8_t)((k < 4 ? qv.x : qv.y) >> ((k & 3) * 8));
+                }
+            }
+            YuvTerms c[8];
+#pragma unroll
+            for (int k = 0; k < 8; k++) c[k] = yuv_chroma(U[k], V[k]);
+#pragma unroll
+            for (int r = 0; r < 2; r++) {
+                const int row = 2 * cy + r;
+                const uint4 qy = __ldg(reinterpret_cast<const uint4 *>(yp + f * fsz + (int64_t)row * w + gx * 16));
+                const uint32_t yw[4] = {qy.x, qy.y, qy.z, qy.w};
+                uint32_t o[12];
+#pragma unroll
+                for (int j = 0; j < 12; j++) o[j] = 0;
+#pragma unroll
+                for (int p = 0; p < 16; p++) {
+                    const int Y = (int)((yw[p >> 2] >> ((p & 3) * 8)) & 0xffu);
+#pragma unroll
+                    for (int ch = 0; ch < 3; ch++) {
+                        const int byte = 3 * p + ch;
+                        o[byte >> 2] |= yuv_px(Y, c[p >> 1], ch) << ((byte & 3) * 8);
+                    }
+                }
+                uint4 *d = reinterpret_cast<uint4 *>(bgr + ((int64_t)f * h * w + (int64_t)row * w + gx * 16) * 3);
+                d[0] = make_uint4(o[0], o[1], o[2], o[3]);
+                d[1] = make_uint4(o[4], o[5], o[6], o[7]);
+                d[2] = make_uint4(o[8], o[9], o[10], o[11]);
+            }
+        }
+    }
+}
+
+int apse_cvt_yuv420_bgr(apse_ctx *ctx, const uint8_t *yuv, int w, int h, int batch, int layout, uint8_t *bgr, void *stream)
+{
+    if (!ctx || !yuv || !bgr || w <= 0 || h <= 0 || (w & 1) || (h & 1) || batch < 1 || layout < APSE_YUV_NV12 || layout > APSE_YUV_YV12)
+        CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "cvt_yuv420_bgr: bad argument (w %d, h %d, batch %d, layout %d)", w, h, batch, layout);
+    const int64_t ysz = (int64_t)w * h, fsz = ysz * 3 / 2;
+    const uint8_t *up, *vp;
+    int cstep, cstride;
+    if (layout == APSE_YUV_NV12 || layout == APSE_YUV_NV21) {
+        up = yuv + ysz + (layout == APSE_YUV_NV21);
+        vp = yuv + ysz + (layout == APSE_YUV_NV12);
+        cstep = 2; cstride = w;
+    } else {   // planar: each chroma plane is (h/2) * (w/2) contiguous bytes (a byte offset: it may start mid-row of a w-wide view)
+        const int64_t csz = ysz / 4;
+        up = yuv + ysz + (layout == APSE_YUV_YV12 ? csz : 0);
+        vp = yuv + ysz + (layout == APSE_YUV_I420 ? csz : 0);
+        cstep = 1; cstride = w / 2;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int gy = batch < 65535 ? batch : 65535;
+    // 16-byte accesses need the caller's buffers 16-byte aligned and rows of whole 16-pixel groups; then every row, chroma row
+    // and frame of the batch starts aligned as well
+    if ((w & 15) == 0 && ((uintptr_t)yuv & 15) == 0 && ((uintptr_t)bgr & 15) == 0) {
+        const int n = (w >> 4) * (h >> 1), gx = div_up(n, 256);
+        if (cstep == 2)
+            KLAUNCH(ctx, KID_YUV2BGR, st, k_yuv420_to_bgr_v16<2><<<dim3(gx, gy), 256, 0, st>>>(yuv, up, vp, cstride, w, h, batch, fsz, bgr));
+        else
+            KLAUNCH(ctx, KID_YUV2BGR, st, k_yuv420_to_bgr_v16<1><<<dim3(gx, gy), 256, 0, st>>>(yuv, up, vp, cstride, w, h, batch, fsz, bgr));
+    } else {
+        const int n = (w >> 1) * (h >> 1), gx = div_up(n, 256);
+        KLAUNCH(ctx, KID_YUV2BGR, st, k_yuv420_to_bgr<<<dim3(gx, gy), 256, 0, st>>>(yuv, up, vp, cstep, cstride, w, h, batch, fsz, bgr));
+    }
+    return APSE_OK;
 }
 
 static int grid_for(const apse_ctx *ctx, int64_t n) { const int64_t cap = (int64_t)ctx->sm_count * 16; return (int)((n + 255) / 256 < cap ? (n + 255) / 256 : cap); }

@@ -168,6 +168,28 @@ class Engine:
             self._check(fn(self.h, src.data_ptr(), npx, dst.data_ptr(), self._stream()))
         return dst
 
+    def cvt_yuv420(self, src, layout, out=None, stream=None):
+        """cv2.cvtColor(src, COLOR_YUV2BGR_<layout>) for layout nv12 / nv21 / i420 / yv12: src [H*3/2, W] or [B, H*3/2, W] uint8
+        (numpy or tensor) -> [.., H, W, 3].  out: a contiguous uint8 CUDA tensor of that shape to write into; stream: torch stream
+        of the launch (None = current)."""
+        torch = self.torch
+        if layout not in _lib.YUV_LAYOUTS:
+            raise ApseError(-1, f"cvt_yuv420: unknown layout {layout!r} (one of {', '.join(_lib.YUV_LAYOUTS)})")
+        src = self._u8(src, "cvtColor")
+        if src.dim() not in (2, 3) or src.shape[-2] % 3:
+            raise ApseError(-1, "cvtColor: YUV 4:2:0 source of shape [H*3/2, W] or [B, H*3/2, W] expected (rows divisible by 3)")
+        rows, W = src.shape[-2:]
+        H = rows * 2 // 3
+        B = src.shape[0] if src.dim() == 3 else 1
+        shape = tuple(src.shape[:-2]) + (H, W, 3)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.uint8, device=self.tdev)
+        elif tuple(out.shape) != shape or out.dtype != torch.uint8 or not out.is_contiguous() or out.device != self.tdev:
+            raise ApseError(-1, f"cvt_yuv420: out must be a contiguous uint8 tensor of shape {shape} on {self.tdev}")
+        st = C.c_void_p(stream.cuda_stream) if stream is not None else self._stream()
+        self._check(self.lib.apse_cvt_yuv420_bgr(self.h, src.data_ptr(), W, H, B, _lib.YUV_LAYOUTS[layout], out.data_ptr(), st))
+        return out
+
     def lut(self, src, lut):
         """cv2.LUT on an arbitrary (possibly strided channel view) uint8 tensor; returns a contiguous tensor."""
         torch = self.torch

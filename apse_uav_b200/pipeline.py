@@ -218,39 +218,72 @@ class Pipeline:
                 self.wait(o)
         return {k: torch.cat([o[k] for o in outs], 0) for k in outs[0]}
 
-    def run_host_stream(self, host_batches, **kw):
+    def _host_staging(self):
+        """The copy stream and the two device BGR staging buffers of the host-frame paths (first use); returns the stream."""
+        if not hasattr(self, "_copy_stream"):
+            torch = self.engine.torch
+            w, h = self.size
+            self._copy_stream = torch.cuda.Stream(device=self.engine.tdev)
+            self._stage = [torch.empty((self.max_batch, h, w, 3), dtype=torch.uint8, device=self.engine.tdev) for _ in range(2)]
+        return self._copy_stream
+
+    def _stage_host_batch(self, hb, i, wait, ready, layout=None):
+        """The host-frame paths' (run_host_stream, shard.run_sequence_host) copy of one pinned host batch into device staging
+        buffer i on the copy stream: after the events `wait` (the last readers of buffer i), then `ready` is recorded.  A BGR
+        batch [b,H,W,3] is copied straight into the buffer.  A YUV 4:2:0 batch [b,H*3/2,W] (layout nv12 / nv21 / i420 / yv12)
+        is copied into a YUV staging buffer (allocated on first use) without waiting and converted into buffer i after the
+        waits: the converted frames then live exactly as long as a BGR batch, which the sparse path needs (it samples the
+        source frames again after the preprocess).  The YUV buffer is free again once its conversion has run, which the copy
+        stream orders, so one is enough.  Returns the staged [b,H,W,3] view."""
+        torch = self.engine.torch
+        dev = self.engine.tdev
+        w, h = self.size
+        cs = self._host_staging()
+        b = int(hb.shape[0])
+        dst = self._stage[i][:b]
+        with torch.cuda.stream(cs):
+            if layout is None:
+                for ev in wait:
+                    cs.wait_event(ev)
+                dst.copy_(hb, non_blocking=True)
+            else:
+                if tuple(hb.shape[1:]) != (h * 3 // 2, w):
+                    raise ApseError(-1, f"{layout} host batches must be [b, {h * 3 // 2}, {w}] uint8, got {tuple(hb.shape)}")
+                if getattr(self, "_yuv_stage", None) is None:
+                    self._yuv_stage = torch.empty((self.max_batch, h * 3 // 2, w), dtype=torch.uint8, device=dev)
+                yuv = self._yuv_stage[:b]
+                yuv.copy_(hb, non_blocking=True)
+                for ev in wait:
+                    cs.wait_event(ev)
+                self.engine.cvt_yuv420(yuv, layout, out=dst, stream=cs)
+            ready.record(cs)
+        return dst
+
+    def run_host_stream(self, host_batches, layout=None, **kw):
         """End-to-end path for frames that live in (pinned) host memory: yields one host result dict per batch.
         Two device staging buffers and a copy stream: the H2D copy of batch k+1 runs while batch k is processed and
-        its detections are read back, so a sequence is bounded by the slower of PCIe and the kernels, not their sum."""
+        its detections are read back, so a sequence is bounded by the slower of PCIe and the kernels, not their sum.
+        layout (None = BGR [b,H,W,3]): "nv12" / "nv21" / "i420" / "yv12" for YUV 4:2:0 batches [b,H*3/2,W] (half the bytes
+        over PCIe), converted on the device as cv2.cvtColor(COLOR_YUV2BGR_<layout>) would."""
         torch = self.engine.torch
         dev = self.engine.tdev
         main = torch.cuda.current_stream(dev)
-        if not hasattr(self, "_copy_stream"):
-            self._copy_stream = torch.cuda.Stream(device=dev)
-            w, h = self.size
-            self._stage = [torch.empty((self.max_batch, h, w, 3), dtype=torch.uint8, device=dev) for _ in range(2)]
-        cs, stage = self._copy_stream, self._stage
         ready = [torch.cuda.Event(), torch.cuda.Event()]
         done = [torch.cuda.Event(), torch.cuda.Event()]
         it = iter(host_batches)
         cur = next(it, None)
         if cur is None:
             return
-        cs.wait_stream(main)
-        with torch.cuda.stream(cs):
-            stage[0][:len(cur)].copy_(cur, non_blocking=True)
-            ready[0].record(cs)
+        self._host_staging().wait_stream(main)
+        staged = [self._stage_host_batch(cur, 0, (), ready[0], layout), None]
         k = 0
         while cur is not None:
             nxt = next(it, None)
             if nxt is not None:
-                if k >= 1:
-                    cs.wait_event(done[(k + 1) % 2])   # the other buffer was the input of batch k-1
-                with torch.cuda.stream(cs):
-                    stage[(k + 1) % 2][:len(nxt)].copy_(nxt, non_blocking=True)
-                    ready[(k + 1) % 2].record(cs)
+                # the other buffer was the input of batch k-1
+                staged[(k + 1) % 2] = self._stage_host_batch(nxt, (k + 1) % 2, [done[(k + 1) % 2]] if k >= 1 else (), ready[(k + 1) % 2], layout)
             main.wait_event(ready[k % 2])
-            det = self.run_batch(stage[k % 2][:len(cur)], **kw)
+            det = self.run_batch(staged[k % 2], **kw)
             done[k % 2].record(main)
             yield self.to_host(det)
             cur, k = nxt, k + 1

@@ -188,10 +188,12 @@ def run_sequence(pipe, frames, rank=0, world=1, group=None, start_frame=1, leds=
 
 
 def run_sequence_host(pipe, host_batches, n_local, rank=0, world=1, group=None, start_frame=1, leds=False, leds_threshold=None,
-                      as_rows=False):
+                      as_rows=False, layout=None):
     """run_sequence for frames that live in (pinned) HOST memory: host_batches yields this rank's block as uint8 tensors
     [b,H,W,3] with b <= pipe.max_batch, n_local frames in total.  Two device staging buffers and a copy stream: the H2D copy
-    of batch k+1 runs under the kernels of batch k; everything after the pipeline is the same as run_sequence."""
+    of batch k+1 runs under the kernels of batch k; everything after the pipeline is the same as run_sequence.
+    layout "nv12" / "nv21" / "i420" / "yv12": the batches are YUV 4:2:0 [b,H*3/2,W] (a video decoder's output, half the bytes
+    of BGR over PCIe), converted on the device as cv2.cvtColor(COLOR_YUV2BGR_<layout>) would (Pipeline._stage_host_batch)."""
     e = pipe.engine
     torch = e.torch
     dev = e.tdev
@@ -199,10 +201,7 @@ def run_sequence_host(pipe, host_batches, n_local, rank=0, world=1, group=None, 
     gray = torch.empty((n_local, h, w), dtype=torch.uint8, device=dev) if leds and n_local else None
     det = e.alloc_detections(n_local, pipe.max_markers, False, pose=True)
     main = torch.cuda.current_stream(dev)
-    if not hasattr(pipe, "_copy_stream"):
-        pipe._copy_stream = torch.cuda.Stream(device=dev)
-        pipe._stage = [torch.empty((pipe.max_batch, h, w, 3), dtype=torch.uint8, device=dev) for _ in range(2)]
-    cs, stage = pipe._copy_stream, pipe._stage
+    cs = pipe._host_staging()
     ready = [torch.cuda.Event(), torch.cuda.Event()]
     free = [None, None]                      # completion events of the batch that last read staging buffer i
     filled = main.record_event()
@@ -213,14 +212,10 @@ def run_sequence_host(pipe, host_batches, n_local, rank=0, world=1, group=None, 
     for k, hb in enumerate(host_batches):
         b = int(hb.shape[0])
         buf = k % 2
-        for ev in free[buf] or ():
-            cs.wait_event(ev)
-        with torch.cuda.stream(cs):
-            stage[buf][:b].copy_(hb, non_blocking=True)
-            ready[buf].record(cs)
+        staged = pipe._stage_host_batch(hb, buf, free[buf] or (), ready[buf], layout)
         main.wait_event(ready[buf])
         sl = {key: v[lo:lo + b] for key, v in det.items()}
-        r = pipe.run_batch(stage[buf][:b], sync=False, input_ready=False, gray_out=None if gray is None else gray[lo:lo + b], out=sl)
+        r = pipe.run_batch(staged, sync=False, input_ready=False, gray_out=None if gray is None else gray[lo:lo + b], out=sl)
         done = list(r.get("_done", ()))
         if not done:
             done = [main.record_event()]

@@ -117,6 +117,14 @@ int apse_cvt_bgr2gray(apse_ctx *ctx, const uint8_t *src, int64_t npx, uint8_t *d
 int apse_lut(apse_ctx *ctx, const uint8_t *src, int64_t n, int src_stride, const uint8_t *lut_dev, uint8_t *dst,
              int dst_stride, void *stream);
 
+/* YUV 4:2:0 layouts of cv2's single-array form [h*3/2][w] (what H.264 / HEVC decoders produce): Y plane, then
+ * NV12: interleaved U V; NV21: interleaved V U; I420 (IYUV): U plane, V plane; YV12: V plane, U plane
+ * (each chroma plane (h/2)*(w/2) contiguous bytes) */
+typedef enum { APSE_YUV_NV12 = 0, APSE_YUV_NV21 = 1, APSE_YUV_I420 = 2, APSE_YUV_YV12 = 3 } apse_yuv_layout;
+/* cv2.cvtColor(src, COLOR_YUV2BGR_{NV12,NV21,I420,YV12}) for a batch: yuv [batch][h*3/2][w], bgr [batch][h][w][3] (device).
+ * w and h even.  Uses no context scratch: the frame size is not bounded by apse_create's max_w / max_h. */
+int apse_cvt_yuv420_bgr(apse_ctx *ctx, const uint8_t *yuv, int w, int h, int batch, int layout, uint8_t *bgr, void *stream);
+
 /* aruco_detect.py:250-259 + :592 fused: remap + Lab gamma + gray for a batch of frames
  * bgr: [batch][h][w][3]; bgr_out (nullable): same shape; gray: [batch][h][w] */
 int apse_preprocess(apse_ctx *ctx, const uint8_t *bgr, uint8_t *bgr_out, uint8_t *gray, int batch, void *stream);

@@ -333,3 +333,41 @@ def make_big_marker_frame(bytes_list, side: int, seed: int = 1, marker_id: int =
     if noise_sigma > 0:
         frame = np.clip(np.rint(frame + rng.normal(0, noise_sigma, frame.shape)), 0, 255).astype(np.uint8)
     return frame
+
+
+# ---- YUV 4:2:0 frames (cv2's single-array form [h*3/2][w]) ------------------------------------------------------------
+def yuv420_from_planes(Y: np.ndarray, U: np.ndarray, V: np.ndarray, layout: str) -> np.ndarray:
+    """Y [h, w], U / V [h/2, w/2] -> [h*3/2, w] in layout nv12 / nv21 / i420 / yv12 (planar chroma planes are contiguous
+    (h/2)*(w/2)-byte runs, so with odd h/2 a plane starts in the middle of a w-wide row, as in cv2)."""
+    h, w = Y.shape
+    if layout in ("nv12", "nv21"):
+        a, b = (U, V) if layout == "nv12" else (V, U)
+        c = np.stack([a, b], -1).reshape(h // 2, w)
+    else:
+        a, b = (U, V) if layout == "i420" else (V, U)
+        c = np.concatenate([a.ravel(), b.ravel()]).reshape(h // 2, w)
+    return np.ascontiguousarray(np.concatenate([Y, c], 0))
+
+
+def bgr_to_yuv420(bgr: np.ndarray, layout: str) -> np.ndarray:
+    """cv2.cvtColor(bgr, COLOR_BGR2YUV_I420), rearranged into `layout` (cv2 has no BGR -> NV12 / NV21 code)"""
+    h, w = bgr.shape[:2]
+    i420 = cv2.cvtColor(bgr, cv2.COLOR_BGR2YUV_I420)
+    flat = i420.reshape(-1)
+    q = (h // 2) * (w // 2)
+    Y, U, V = flat[:h * w].reshape(h, w), flat[h * w:h * w + q].reshape(h // 2, w // 2), flat[h * w + q:].reshape(h // 2, w // 2)
+    return yuv420_from_planes(Y, U, V, layout)
+
+
+def yuv420_all_triples(layout: str) -> np.ndarray:
+    """A 4096 x 4096 frame holding every (Y, U, V) triple once: 2x2 block b carries the (U, V) pair b // 64 and the four Y
+    values 4 (b % 64) .. 4 (b % 64) + 3, so the 64 blocks of a pair enumerate all 256 Y values."""
+    n = 2048
+    b = np.arange(n * n, dtype=np.int64).reshape(n, n)
+    pair, yq = b // 64, b % 64
+    U, V = (pair >> 8).astype(np.uint8), (pair & 255).astype(np.uint8)
+    Y = np.empty((2 * n, 2 * n), np.uint8)
+    for dy in (0, 1):
+        for dx in (0, 1):
+            Y[dy::2, dx::2] = (4 * yq + 2 * dy + dx).astype(np.uint8)
+    return yuv420_from_planes(Y, U, V, layout)
