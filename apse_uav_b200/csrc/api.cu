@@ -8,6 +8,12 @@
 int apse_upload_tables(apse_ctx *ctx, const uint8_t *lut, LabTables **dev, cudaStream_t st);  // preprocess.cu
 int apse_upload_p2_tables(apse_ctx *ctx, const uint8_t *lut, P2Tables **dev, cudaStream_t st);
 
+// cached tile extrema (apse_preprocess_tiles) never survive another entry point
+static void drop_handoffs(apse_ctx *ctx) { for (TileSlot &s : ctx->slot) s.gray = nullptr; }
+
+// the slot the last apse_preprocess_tiles[_sparse] call filled
+static TileSlot &last_slot(apse_ctx *ctx) { return ctx->slot[ctx->next_slot ^ 1]; }
+
 extern "C" {
 
 int apse_abi_version(void) { return APSE_ABI_VERSION; }
@@ -133,7 +139,7 @@ int apse_set_camera(apse_ctx *ctx, const double K[9], const double D[14], int w,
     }
     int rc = apse_init_undistort_map(ctx, K, D, w, h, ctx->mapx, ctx->mapy, stream);
     if (rc) return rc;
-    ctx->tiles_gray[0] = ctx->tiles_gray[1] = nullptr;   // cached tile extrema (apse_preprocess_tiles) never survive another entry point
+    drop_handoffs(ctx);
     memcpy(ctx->K, K, sizeof ctx->K);
     memcpy(ctx->D, D, sizeof ctx->D);
     ctx->w = w; ctx->h = h;
@@ -145,7 +151,7 @@ int apse_set_lut(apse_ctx *ctx, const uint8_t lut[256], void *stream)
 {
     if (!ctx || !lut) CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "set_lut: bad argument");
     memcpy(ctx->lut, lut, 256);
-    ctx->tiles_gray[0] = ctx->tiles_gray[1] = nullptr;   // cached tile extrema (apse_preprocess_tiles) never survive another entry point
+    drop_handoffs(ctx);
     int rc = apse_upload_tables(ctx, lut, &ctx->tables, (cudaStream_t)stream);
     if (rc) return rc;
     rc = apse_upload_p2_tables(ctx, lut, &ctx->tables2, (cudaStream_t)stream);
@@ -192,7 +198,7 @@ int apse_set_params(apse_ctx *ctx, const apse_params *p)
     if (p->cornerRefinementMethod < 0 || p->cornerRefinementMethod > 3) CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "set_params: cornerRefinementMethod must be 0 .. 3");
     if (p->aprilTagMaxNmaxima < 4 || p->aprilTagMaxNmaxima > 16)
         CTX_FAIL(ctx, APSE_ERR_UNSUPPORTED, "set_params: aprilTagMaxNmaxima must be in [4,16]");
-    ctx->tiles_gray[0] = ctx->tiles_gray[1] = nullptr;   // cached tile extrema (apse_preprocess_tiles) never survive another entry point
+    drop_handoffs(ctx);
     ctx->params = *p;
     ctx->has_params = true;
     return APSE_OK;
@@ -274,13 +280,16 @@ int apse_fill_device_params(apse_ctx *ctx, DeviceParams *dp, int w, int h)
     return APSE_OK;
 }
 
-// candidates (APRILTAG quad detector or the classic threshold / contour path) -> grouping + decoding -> SUBPIX
+// candidates (APRILTAG quad detector or the classic threshold / contour path) -> grouping + decoding -> SUBPIX.  tiles: the slot
+// holding this batch's tile extrema (and, for a sparse batch, its flags), or null.  Extrema the chain computes itself go to the
+// handed slot (the only one it writes: Pipeline), else to slot 0 (the caller orders the call against pending work on the context).
 static int apse_detect_impl(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, apse_detections *out, cudaStream_t st,
-                            bool have_tile_minmax)
+                            const TileSlot *tiles)
 {
     DeviceParams dp;
     apse_fill_device_params(ctx, &dp, w, h);
     const int mode = ctx->params.cornerRefinementMethod;
+    uint16_t *tmm_scratch = (tiles ? tiles : &ctx->slot[0])->tmm;
     // both candidate paths can produce more than DEC_SMEMC candidates per frame (a 4K frame with a few hundred small markers
     // does on the APRILTAG path): the decode stage then needs its global candidate arrays, whatever ran on the context before
     int rc = apse_decode_big_scratch(ctx);
@@ -293,19 +302,50 @@ static int apse_detect_impl(apse_ctx *ctx, const uint8_t *gray, int w, int h, in
         if (rc) return rc;
         DeviceParams dq;
         apse_fill_device_params(ctx, &dq, qw, qh);
-        rc = apse_apriltag_quads(ctx, qim, qw, qh, batch, dq, st, false);
+        rc = apse_apriltag_quads(ctx, qim, qw, qh, batch, dq, st, nullptr, tmm_scratch);
         if (!rc && qscale != 1.f) rc = apse_scale_quads(ctx, batch, qscale, st);
     } else if (mode == 3) {
-        rc = apse_apriltag_quads(ctx, gray, w, h, batch, dp, st, have_tile_minmax);
+        rc = apse_apriltag_quads(ctx, gray, w, h, batch, dp, st, tiles, tmm_scratch);
     } else {
         rc = apse_classic_quads(ctx, gray, w, h, batch, st);
     }
     if (rc) return rc;
-    rc = apse_decode_candidates(ctx, gray, w, h, batch, dp, out, st);
+    SparseSrc sparse;
+    if (tiles && tiles->bgr) sparse = SparseSrc{tiles->bgr, ctx->mapx, ctx->mapy, ctx->tables2, tiles->eflag, w / 4, h / 4};
+    rc = apse_decode_candidates(ctx, gray, w, h, batch, dp, tiles && tiles->bgr ? &sparse : nullptr, out, st);
     if (rc) return rc;
     if (mode == 1) rc = apse_corner_subpix(ctx, gray, w, h, batch, out, st);
     if (mode == 2) rc = apse_contour_refine(ctx, batch, out, st);
     return rc;
+}
+
+static int detect_pose(apse_ctx *ctx, const uint8_t *gray, int batch, const TileSlot *tiles, apse_detections *out, const float *marker_len,
+                       float marker_len_all, double *rvec, double *tvec, void *stream)
+{
+    int rc = apse_detect_impl(ctx, gray, ctx->w, ctx->h, batch, out, (cudaStream_t)stream, tiles);
+    if (rc) return rc;
+    if (rvec && tvec)
+        rc = apse_pose_frames(ctx, out->corners, out->n_markers, batch, out->max_markers, marker_len, marker_len_all, ctx->K, ctx->D, rvec, tvec, stream);
+    return rc;
+}
+
+// K1 writes the 4x4-tile extrema of gray straight into the slot, for the candidate stage.  want_sparse: the caller does not need
+// the gray frames, so they may come from the sparse evaluation (identical detections; gray is computed only where the detector
+// reads it).  On return slot.gray says whether extrema were produced.
+static int preprocess_into(apse_ctx *ctx, TileSlot &slot, const uint8_t *bgr, uint8_t *gray, int batch, cudaStream_t st, bool want_sparse)
+{
+    int rc = 1;
+    slot.bgr = nullptr;
+    if (want_sparse && ctx->params.cornerRefinementMethod == 3 && !apse_quad_image_needed(ctx->params)) {
+        rc = apse_preprocess_sparse(ctx, slot, bgr, gray, batch, ctx->params.aprilTagMinWhiteBlackDiff, st);
+        if (rc < 0) return rc;
+        if (rc == APSE_OK) slot.bgr = bgr;
+    }
+    if (rc == 1) rc = apse_preprocess_ex(ctx, bgr, nullptr, gray, slot.tmm, batch, st);
+    if (rc < 0) return rc;
+    slot.gray = rc == APSE_OK ? gray : nullptr;
+    slot.batch = batch;
+    return APSE_OK;
 }
 
 extern "C" {
@@ -314,8 +354,8 @@ int apse_detect(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, aps
 {
     if (!ctx || !gray || !out || batch <= 0) CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "detect: bad argument");
     if (!ctx->has_dict) CTX_FAIL(ctx, APSE_ERR_NOT_CONFIGURED, "detect: set_dictionary first");
-    ctx->tiles_gray[0] = ctx->tiles_gray[1] = nullptr;   // cached tile extrema (apse_preprocess_tiles) never survive another entry point
-    return apse_detect_impl(ctx, gray, w, h, batch, out, (cudaStream_t)stream, false);
+    drop_handoffs(ctx);
+    return apse_detect_impl(ctx, gray, w, h, batch, out, (cudaStream_t)stream, nullptr);
 }
 
 int apse_process_frames(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gray, int batch, apse_detections *out, const float *marker_len,
@@ -325,36 +365,19 @@ int apse_process_frames(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gray, int ba
     if (!ctx->has_camera || !ctx->has_lut || !ctx->has_dict)
         CTX_FAIL(ctx, APSE_ERR_NOT_CONFIGURED, "process_frames: set_camera, set_lut and set_dictionary first");
     if (batch > ctx->max_batch) CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "process_frames: batch %d exceeds the context capacity %d", batch, ctx->max_batch);
-    ctx->tiles_gray[0] = ctx->tiles_gray[1] = nullptr;   // cached tile extrema (apse_preprocess_tiles) never survive another entry point
-    cudaStream_t st = (cudaStream_t)stream;
-    const int w = ctx->w, h = ctx->h;
+    drop_handoffs(ctx);
     const bool want_sparse = gray == nullptr;
     if (!gray) {
         if (!ctx->gray_scratch) CUDA_TRY(ctx, cudaMalloc((void **)&ctx->gray_scratch, (size_t)ctx->max_batch * ctx->max_w * ctx->max_h));
         gray = ctx->gray_scratch;
     }
-    // K1 writes the 4x4-tile extrema of gray straight into the candidate stage's tile arrays.  A caller that does not ask for
-    // the gray frames gets the sparse evaluation (identical detections; gray is computed only where the detector reads it).
-    int rc = 1;
-    const bool sparse = want_sparse && ctx->params.cornerRefinementMethod == 3 && !apse_quad_image_needed(ctx->params);
-    if (sparse) {
-        rc = apse_preprocess_sparse(ctx, bgr, gray, ctx->tmm, 0, batch, ctx->params.aprilTagMinWhiteBlackDiff, st);
-        if (rc < 0) return rc;
-        if (rc == APSE_OK) {
-            ctx->sparse_active = true;
-            ctx->sparse_src = SparseSrc{bgr, ctx->mapx, ctx->mapy, ctx->tables2, ctx->eflag[0], w / 4, h / 4};
-            ctx->sparse_elist = ctx->elist[0]; ctx->sparse_ecount = ctx->ecount[0];
-        }
-    }
-    if (rc == 1) rc = apse_preprocess_ex(ctx, bgr, nullptr, gray, ctx->tmm, batch, st);
-    if (rc < 0) return rc;
-    const bool have_minmax = rc == APSE_OK;
-    rc = apse_detect_impl(ctx, gray, w, h, batch, out, st, have_minmax);
-    ctx->sparse_active = false;
+    // slot 0 on the caller's stream, handed straight to the detector; the refusal records (partial_gray) are left as they are
+    TileSlot &slot = ctx->slot[0];
+    int rc = preprocess_into(ctx, slot, bgr, gray, batch, (cudaStream_t)stream, want_sparse);
     if (rc) return rc;
-    if (rvec && tvec)
-        rc = apse_pose_frames(ctx, out->corners, out->n_markers, batch, out->max_markers, marker_len, marker_len_all, ctx->K, ctx->D, rvec, tvec, stream);
-    return rc;
+    const bool have_extrema = slot.gray != nullptr;
+    slot.gray = nullptr;
+    return detect_pose(ctx, gray, batch, have_extrema ? &slot : nullptr, out, marker_len, marker_len_all, rvec, tvec, stream);
 }
 
 static int preprocess_tiles_impl(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gray, int batch, void *stream, bool want_sparse)
@@ -362,23 +385,12 @@ static int preprocess_tiles_impl(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gra
     if (!ctx || !bgr || !gray || batch <= 0) CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "preprocess_tiles: bad argument");
     if (!ctx->has_camera || !ctx->has_lut) CTX_FAIL(ctx, APSE_ERR_NOT_CONFIGURED, "preprocess_tiles: set_camera and set_lut first");
     if (batch > ctx->max_batch) CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "preprocess_tiles: batch %d exceeds the context capacity %d", batch, ctx->max_batch);
-    // two tile-extrema buffers: the preprocess of the next sub-batch may run while the chain of the previous one (which
-    // reads its own buffer) is still in flight; the caller alternates the gray buffers accordingly (Pipeline)
-    const int slot = ctx->tiles_slot;
-    ctx->tiles_slot ^= 1;
-    int rc = 1;
-    ctx->tiles_sparse[slot] = false;
-    for (int k = 0; k < 2; k++) if (ctx->sparse_gray[k] == gray) ctx->sparse_gray[k] = nullptr;   // the buffer is rewritten now
-    if (want_sparse && ctx->params.cornerRefinementMethod == 3 && !apse_quad_image_needed(ctx->params)) {
-        rc = apse_preprocess_sparse(ctx, bgr, gray, ctx->tmm_buf[slot], slot, batch, ctx->params.aprilTagMinWhiteBlackDiff, (cudaStream_t)stream);
-        if (rc < 0) return rc;
-        if (rc == APSE_OK) { ctx->tiles_sparse[slot] = true; ctx->tiles_bgr[slot] = bgr; ctx->sparse_gray[slot] = gray; }
-    }
-    if (rc == 1) rc = apse_preprocess_ex(ctx, bgr, nullptr, gray, ctx->tmm_buf[slot], batch, (cudaStream_t)stream);
-    if (rc < 0) return rc;
-    ctx->tiles_gray[slot] = rc == APSE_OK ? gray : nullptr;   // the extrema in tmm_buf[slot] belong to exactly this gray batch
-    ctx->tiles_batch[slot] = batch;
-    return APSE_OK;
+    TileSlot &slot = ctx->slot[ctx->next_slot];
+    ctx->next_slot ^= 1;
+    for (TileSlot &s : ctx->slot) if (s.partial_gray == gray) s.partial_gray = nullptr;   // the buffer is rewritten now
+    int rc = preprocess_into(ctx, slot, bgr, gray, batch, (cudaStream_t)stream, want_sparse);
+    if (!rc && slot.bgr) slot.partial_gray = gray;
+    return rc;
 }
 
 int apse_preprocess_tiles(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gray, int batch, void *stream)
@@ -396,31 +408,19 @@ int apse_detect_pose_frames(apse_ctx *ctx, const uint8_t *gray, int batch, apse_
 {
     if (!ctx || !gray || !out || batch <= 0) CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "detect_pose_frames: bad argument");
     if (!ctx->has_camera || !ctx->has_dict) CTX_FAIL(ctx, APSE_ERR_NOT_CONFIGURED, "detect_pose_frames: set_camera and set_dictionary first");
-    bool have_minmax = false;
-    for (int slot = 0; slot < 2 && !have_minmax; slot++)
-        if (ctx->tiles_gray[slot] == gray && ctx->tiles_batch[slot] == batch) {
-            have_minmax = true;
-            ctx->tmm = ctx->tmm_buf[slot];
-            ctx->tiles_gray[slot] = nullptr;              // consumed: a later call on other data recomputes the extrema
-            if (ctx->tiles_sparse[slot]) {
-                ctx->sparse_active = true;
-                ctx->sparse_src = SparseSrc{ctx->tiles_bgr[slot], ctx->mapx, ctx->mapy, ctx->tables2, ctx->eflag[slot], ctx->w / 4, ctx->h / 4};
-                ctx->sparse_elist = ctx->elist[slot]; ctx->sparse_ecount = ctx->ecount[slot];
-                ctx->tiles_sparse[slot] = false;
-                ctx->sparse_gray[slot] = nullptr;
-            }
-        }
-    // a gray batch of the sparse evaluation is only complete together with its tile flags: without them (another entry point
-    // came in between) the detector would read pixels that were never computed
-    if (!have_minmax && (ctx->sparse_gray[0] == gray || ctx->sparse_gray[1] == gray))
+    TileSlot *tiles = nullptr;
+    for (TileSlot &s : ctx->slot)
+        if (!tiles && s.gray == gray && s.batch == batch) tiles = &s;
+    if (tiles) {
+        tiles->gray = nullptr;                         // consumed: a later call on other data recomputes the extrema
+        if (tiles->bgr) tiles->partial_gray = nullptr;
+    } else if (ctx->slot[0].partial_gray == gray || ctx->slot[1].partial_gray == gray) {
+        // a gray batch of the sparse evaluation is only complete together with its tile flags: without them (another entry
+        // point came in between) the detector would read pixels that were never computed
         CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "detect_pose_frames: this gray batch comes from apse_preprocess_tiles_sparse and its tile flags are gone "
                                             "(another call on the context came in between); preprocess it again");
-    int rc = apse_detect_impl(ctx, gray, ctx->w, ctx->h, batch, out, (cudaStream_t)stream, have_minmax);
-    ctx->sparse_active = false;
-    if (rc) return rc;
-    if (rvec && tvec)
-        rc = apse_pose_frames(ctx, out->corners, out->n_markers, batch, out->max_markers, marker_len, marker_len_all, ctx->K, ctx->D, rvec, tvec, stream);
-    return rc;
+    }
+    return detect_pose(ctx, gray, batch, tiles, out, marker_len, marker_len_all, rvec, tvec, stream);
 }
 
 int apse_adaptive_threshold(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, int win, double c, uint8_t *out, void *stream)
@@ -468,11 +468,11 @@ int apse_debug_sparse(apse_ctx *ctx, uint16_t *bound_table_host, uint8_t *eflag_
         CUDA_TRY(ctx, cudaMemcpyAsync(bound_table_host, ctx->btable, 16 * 32 * 32 * sizeof(uint16_t), cudaMemcpyDeviceToHost, st));
         CUDA_TRY(ctx, cudaStreamSynchronize(st));
     }
-    const int slot = ctx->tiles_slot ^ 1;   // the slot the last apse_preprocess_tiles[_sparse] call used
+    const TileSlot &slot = last_slot(ctx);
     if (eflag_dev || n_exact_host) {
-        if (!ctx->eflag[slot]) CTX_FAIL(ctx, APSE_ERR_NOT_CONFIGURED, "debug_sparse: no sparse batch was preprocessed on this context");
-        if (eflag_dev) CUDA_TRY(ctx, cudaMemcpyAsync(eflag_dev, ctx->eflag[slot], (size_t)batch * (ctx->w / 4) * (ctx->h / 4), cudaMemcpyDeviceToDevice, st));
-        if (n_exact_host) CUDA_TRY(ctx, cudaMemcpyAsync(n_exact_host, ctx->ecount[slot], sizeof(int), cudaMemcpyDeviceToHost, st));
+        if (!slot.eflag) CTX_FAIL(ctx, APSE_ERR_NOT_CONFIGURED, "debug_sparse: no sparse batch was preprocessed on this context");
+        if (eflag_dev) CUDA_TRY(ctx, cudaMemcpyAsync(eflag_dev, slot.eflag, (size_t)batch * (ctx->w / 4) * (ctx->h / 4), cudaMemcpyDeviceToDevice, st));
+        if (n_exact_host) CUDA_TRY(ctx, cudaMemcpyAsync(n_exact_host, slot.ecount, sizeof(int), cudaMemcpyDeviceToHost, st));
         CUDA_TRY(ctx, cudaStreamSynchronize(st));
     }
     return APSE_OK;
@@ -481,9 +481,9 @@ int apse_debug_sparse(apse_ctx *ctx, uint16_t *bound_table_host, uint8_t *eflag_
 int apse_debug_tile_bounds(apse_ctx *ctx, uint16_t *bounds_dev, int batch, void *stream)
 {
     if (!ctx || !bounds_dev || batch <= 0 || batch > ctx->max_batch) CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "debug_tile_bounds: bad argument");
-    const int slot = ctx->tiles_slot ^ 1;   // the slot the last apse_preprocess_tiles[_sparse] call used
-    if (!ctx->tbounds[slot]) CTX_FAIL(ctx, APSE_ERR_NOT_CONFIGURED, "debug_tile_bounds: no sparse batch was preprocessed on this context");
-    CUDA_TRY(ctx, cudaMemcpyAsync(bounds_dev, ctx->tbounds[slot], (size_t)batch * (ctx->w / 4) * (ctx->h / 4) * sizeof(uint16_t),
+    const TileSlot &slot = last_slot(ctx);
+    if (!slot.tbounds) CTX_FAIL(ctx, APSE_ERR_NOT_CONFIGURED, "debug_tile_bounds: no sparse batch was preprocessed on this context");
+    CUDA_TRY(ctx, cudaMemcpyAsync(bounds_dev, slot.tbounds, (size_t)batch * (ctx->w / 4) * (ctx->h / 4) * sizeof(uint16_t),
                                   cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     return APSE_OK;
 }
@@ -491,11 +491,10 @@ int apse_debug_tile_bounds(apse_ctx *ctx, uint16_t *bounds_dev, int batch, void 
 int apse_debug_tile_extrema(apse_ctx *ctx, uint16_t *dst_dev, int batch, void *stream)
 {
     if (!ctx || !dst_dev || batch <= 0 || batch > ctx->max_batch) CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "debug_tile_extrema: bad argument");
-    const int slot = ctx->tiles_slot ^ 1;   // the slot the last apse_preprocess_tiles[_sparse] call used
-    // tiles_gray[slot] is set only when that call produced extrema, and cleared by any call that drops them
-    if (!ctx->tiles_gray[slot]) CTX_FAIL(ctx, APSE_ERR_NOT_CONFIGURED, "debug_tile_extrema: the last preprocess_tiles batch left no tile extrema");
-    if (batch > ctx->tiles_batch[slot]) CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "debug_tile_extrema: batch %d exceeds the preprocessed batch %d", batch, ctx->tiles_batch[slot]);
-    CUDA_TRY(ctx, cudaMemcpyAsync(dst_dev, ctx->tmm_buf[slot], (size_t)batch * (ctx->w / 4) * (ctx->h / 4) * sizeof(uint16_t),
+    const TileSlot &slot = last_slot(ctx);
+    if (!slot.gray) CTX_FAIL(ctx, APSE_ERR_NOT_CONFIGURED, "debug_tile_extrema: the last preprocess_tiles batch left no tile extrema");
+    if (batch > slot.batch) CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "debug_tile_extrema: batch %d exceeds the preprocessed batch %d", batch, slot.batch);
+    CUDA_TRY(ctx, cudaMemcpyAsync(dst_dev, slot.tmm, (size_t)batch * (ctx->w / 4) * (ctx->h / 4) * sizeof(uint16_t),
                                   cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     return APSE_OK;
 }
@@ -507,7 +506,7 @@ int apse_debug_apriltag(apse_ctx *ctx, const uint8_t *gray, int w, int h, uint8_
     cudaStream_t st = (cudaStream_t)stream;
     DeviceParams dp;
     apse_fill_device_params(ctx, &dp, w, h);
-    int rc = apse_apriltag_quads(ctx, gray, w, h, 1, dp, st, false, true);
+    int rc = apse_apriltag_quads(ctx, gray, w, h, 1, dp, st, nullptr, ctx->slot[0].tmm, true);
     if (rc) return rc;
     size_t npx = (size_t)w * h;
     if (thresh) CUDA_TRY(ctx, cudaMemcpyAsync(thresh, ctx->thresh, npx, cudaMemcpyDeviceToDevice, st));

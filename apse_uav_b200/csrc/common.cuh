@@ -72,6 +72,28 @@ enum KernelId {
 };
 #define APSE_EVENT_POOL 2048
 
+// One preprocess -> detect hand-off (api.cu).  apse_preprocess_tiles[_sparse] fills the two slots in turn, so that the preprocess
+// of the next sub-batch can run while the chain of the previous one still reads its own slot (Pipeline alternates its two gray
+// buffers to match); apse_detect_pose_frames consumes the slot whose gray and batch it is handed.  apse_process_frames runs
+// through slot 0 and hands nothing on.  Rules:
+//   * extrema serve one detect call, on exactly the gray batch they were computed with;
+//   * cached extrema never survive another entry point: the setters, apse_detect and apse_process_frames drop every hand-off;
+//   * a sparse gray batch is exact only on the tiles its slot flags, so it must not reach the detector without them:
+//     partial_gray refuses it after its hand-off was dropped.
+struct TileSlot {
+    uint16_t *tmm = nullptr;          // [max_batch][h/4][w/4] 4x4-tile extrema of gray, min | max << 8
+    // sparse evaluation buffers (first use): per-tile bounds of gray (lo | hi << 8), 1 = tile evaluated exactly, the list of
+    // those tiles (ATILE entries, capacity = every tile of the batch) and its length
+    uint16_t *tbounds = nullptr;
+    uint8_t *eflag = nullptr;
+    uint32_t *elist = nullptr;
+    int *ecount = nullptr;
+    const uint8_t *gray = nullptr;    // gray batch the extrema belong to; null = none (not produced, consumed or dropped)
+    int batch = 0;
+    const uint8_t *bgr = nullptr;     // non-null: sparse batch (gray exact only on the eflag tiles), its source frames
+    const uint8_t *partial_gray = nullptr;   // gray written sparsely for this slot and not rewritten since
+};
+
 struct apse_ctx {
     int device = 0, max_w = 0, max_h = 0, max_batch = 0;
     int sm_count = 148;               // queried at apse_create; persistent grids are sized in multiples of it
@@ -106,8 +128,8 @@ struct apse_ctx {
     apse_params params;
     // APRILTAG scratch (sized for max_batch frames of max_w x max_h)
     uint8_t *thresh = nullptr;
-    uint16_t *tmm = nullptr;          // 4x4-tile extrema of gray, min | max << 8, [batch][h/4][w/4] (= one of tmm_buf)
-    uint16_t *tmm_buf[2] = {nullptr, nullptr};   // apse_preprocess_tiles alternates between them
+    TileSlot slot[2];
+    int next_slot = 0;                // the slot the next apse_preprocess_tiles[_sparse] call fills
     uint32_t *labels = nullptr;
     uint4 *points = nullptr;          // {key_lo, key_hi, xy, slot|g}
     uint32_t *point_rank = nullptr;
@@ -124,27 +146,14 @@ struct apse_ctx {
     uint32_t *quad_order = nullptr;   // rank of each quad in the dependency's candidate order (apse_rank_quads)
     // decode scratch
     void *decode_scratch = nullptr;
-    const uint8_t *tiles_gray[2] = {nullptr, nullptr};   // gray batch whose tile extrema are in tmm_buf[i] (apse_preprocess_tiles -> apse_detect_pose_frames)
-    int tiles_batch[2] = {0, 0}, tiles_slot = 0;
     uint8_t *nbr_mask = nullptr;      // [max_batch][h][w] 8-neighbour foreground masks of the classic path (first use)
     uint8_t *gray_scratch = nullptr;  // [max_batch][h][w], allocated on first use by apse_process_frames(gray = NULL)
     void *seq_jobs = nullptr, *seq_results = nullptr;   // device staging of apse_sequence_jobs (grown on demand)
     int seq_cap = 0;
-    // sparse evaluation (apse_preprocess_tiles_sparse / apse_process_frames without a gray output), one set per tiles slot
+    // sparse evaluation (apse_preprocess_tiles_sparse / apse_process_frames without a gray output); its buffers are per TileSlot
     uint16_t *btable = nullptr;       // [SB_ENTRIES] bound table: min | (255 - max) << 8 of gray over the colours of a cell
     cudaStream_t aux_stream = nullptr;   // high-priority stream of the flag / exact kernels of a sparse batch (first use)
     cudaEvent_t aux_ev[2] = {nullptr, nullptr};
-    uint16_t *tbounds[2] = {nullptr, nullptr};   // [max_batch][h/4][w/4] per-tile bounds of gray (lo | hi << 8)
-    uint8_t *eflag[2] = {nullptr, nullptr};      // [max_batch][h/4][w/4] 1 = tile evaluated exactly
-    uint32_t *elist[2] = {nullptr, nullptr};     // tiles to evaluate exactly (ATILE entries), capacity = every tile of the batch
-    int *ecount[2] = {nullptr, nullptr};
-    const uint8_t *tiles_bgr[2] = {nullptr, nullptr};   // source frames of the batch in slot i (sparse batches only)
-    bool tiles_sparse[2] = {false, false};
-    const uint8_t *sparse_gray[2] = {nullptr, nullptr};   // gray buffer a sparse batch was written into (partial: only valid with its slot)
-    bool sparse_active = false;       // the detect call in flight reads gray through sparse_src
-    SparseSrc sparse_src;
-    const uint32_t *sparse_elist = nullptr;   // tiles of that batch that carry exact extrema (k_threshold_scan_list)
-    const int *sparse_ecount = nullptr;
     // image of the quad detector when aprilTagQuadDecimate / aprilTagQuadSigma are set (quadim.cu), allocated on first use
     uint32_t *trace_strips = nullptr; // classic path: per-warp temporary point strips of k_trace_long
     size_t trace_strips_bytes = 0;
@@ -209,10 +218,9 @@ static __host__ __device__ inline int div_up(int a, int b) { return (a + b - 1) 
 // internal entry points implemented per translation unit
 int apse_preprocess_ex(apse_ctx *ctx, const uint8_t *bgr, uint8_t *bgr_out, uint8_t *gray, uint16_t *tmm, int batch,
                        cudaStream_t st);   // returns 1 when the tile extrema were not produced (generic path)
-// sparse evaluation: bounds pass + flags + exact chain on the flagged tiles; fills tmm and ctx->eflag[slot].  Returns 1 when the
-// frame geometry has no TMA path (the caller falls back to the dense kernel)
-int apse_preprocess_sparse(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gray, uint16_t *tmm, int slot, int batch, int min_wb_diff,
-                           cudaStream_t st);
+// sparse evaluation: bounds pass + flags + exact chain on the flagged tiles; fills the slot's tmm and sparse buffers.  Returns 1
+// when the frame geometry has no TMA path (the caller falls back to the dense kernel)
+int apse_preprocess_sparse(apse_ctx *ctx, TileSlot &slot, const uint8_t *bgr, uint8_t *gray, int batch, int min_wb_diff, cudaStream_t st);
 int apse_build_bound_table(apse_ctx *ctx, cudaStream_t st);
 bool apse_quad_image_needed(const apse_params &p);
 int apse_quad_image(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, const uint8_t **out, int *qw, int *qh, float *scale, cudaStream_t st);
@@ -223,9 +231,11 @@ void apse_detect_free(apse_ctx *ctx);
 int apse_decode_alloc(apse_ctx *ctx);
 void apse_decode_free(apse_ctx *ctx);
 int apse_fill_device_params(apse_ctx *ctx, DeviceParams *dp, int w, int h);
-int apse_apriltag_quads(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, const DeviceParams &dp,
-                        cudaStream_t st, bool have_tile_minmax = false,    // true: ctx->tmm already holds this batch's tile extrema
-                        bool flat_labels = false);                         // true: ctx->labels fully flattened (debug entry point)
+// tiles: the slot holding this batch's tile extrema (and, for a sparse batch, the flags of its exact tiles), or null: the extrema
+// are computed into tmm_scratch
+int apse_apriltag_quads(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, const DeviceParams &dp, cudaStream_t st,
+                        const TileSlot *tiles, uint16_t *tmm_scratch,
+                        bool flat_labels = false);   // true: ctx->labels fully flattened (debug entry point)
 int apse_decode_big_scratch(apse_ctx *ctx);
 int apse_adaptive_threshold_impl(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, int win, double c, uint8_t *out, cudaStream_t st);
 int apse_classic_quads(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, cudaStream_t st);
@@ -234,5 +244,6 @@ int apse_contour_refine(apse_ctx *ctx, int batch, apse_detections *out, cudaStre
 int apse_corner_subpix(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, apse_detections *out, cudaStream_t st);
 int apse_decode_tap(apse_ctx *ctx, const uint8_t *gray, int w, int h, const float *corners, int n, const DeviceParams &dp, uint8_t *img_out,
                     uint8_t *bits_out, int32_t *res_out, cudaStream_t st);
+// sparse: how to compute the pixels of a sparse gray batch that were not evaluated, or null (dense gray)
 int apse_decode_candidates(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, const DeviceParams &dp,
-                           apse_detections *out, cudaStream_t st);
+                           const SparseSrc *sparse, apse_detections *out, cudaStream_t st);

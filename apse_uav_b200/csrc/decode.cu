@@ -802,7 +802,7 @@ int apse_decode_big_scratch(apse_ctx *ctx)
 }
 
 int apse_decode_candidates(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, const DeviceParams &dp,
-                           apse_detections *out, cudaStream_t st)
+                           const SparseSrc *sparse, apse_detections *out, cudaStream_t st)
 {
     if (!out || !out->corners || !out->ids || !out->n_markers || !out->status || out->max_markers <= 0)
         CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "detect: incomplete apse_detections");
@@ -814,8 +814,8 @@ int apse_decode_candidates(apse_ctx *ctx, const uint8_t *gray, int w, int h, int
     // hierarchy scratch of the quad fit is free at this point: [batch][APSE_MAX_QUADS] decode results
     int32_t *dec_raw = reinterpret_cast<int32_t *>(ctx->errs);
     const int cand_blocks = ctx->params.cornerRefinementMethod == 3 ? 64 : 512;   // CTAs per frame; a CTA without a candidate exits at once
-    if (ctx->sparse_active)
-        KLAUNCH(ctx, KID_DECODE_BITS, st, k_decode_bits<true><<<dim3(cand_blocks, batch), DECB_THREADS, 0, st>>>(gray, w, h, ctx->quads, ctx->counters, dp, ctx->dict, dec_raw, ctx->sparse_src));
+    if (sparse)
+        KLAUNCH(ctx, KID_DECODE_BITS, st, k_decode_bits<true><<<dim3(cand_blocks, batch), DECB_THREADS, 0, st>>>(gray, w, h, ctx->quads, ctx->counters, dp, ctx->dict, dec_raw, *sparse));
     else
         KLAUNCH(ctx, KID_DECODE_BITS, st, k_decode_bits<false><<<dim3(cand_blocks, batch), DECB_THREADS, 0, st>>>(gray, w, h, ctx->quads, ctx->counters, dp, ctx->dict, dec_raw, SparseSrc{}));
     // the classic path (hundreds of candidates per frame) launches with the shared memory of the middle tier; the APRILTAG path keeps

@@ -1214,8 +1214,7 @@ int apse_detect_alloc(apse_ctx *ctx)
     size_t B = ctx->max_batch, npx = (size_t)ctx->max_w * ctx->max_h;
     size_t ntiles = (size_t)div_up(ctx->max_w, 4) * div_up(ctx->max_h, 4);
     CUDA_TRY(ctx, cudaMalloc((void **)&ctx->thresh, B * npx));
-    for (int k = 0; k < 2; k++) CUDA_TRY(ctx, cudaMalloc((void **)&ctx->tmm_buf[k], B * ntiles * sizeof(uint16_t)));
-    ctx->tmm = ctx->tmm_buf[0];
+    for (TileSlot &s : ctx->slot) CUDA_TRY(ctx, cudaMalloc((void **)&s.tmm, B * ntiles * sizeof(uint16_t)));
     CUDA_TRY(ctx, cudaMalloc((void **)&ctx->labels, B * npx * sizeof(uint32_t)));
     CUDA_TRY(ctx, cudaMalloc((void **)&ctx->points, B * APSE_MAX_POINTS * sizeof(uint4)));
     CUDA_TRY(ctx, cudaMalloc((void **)&ctx->hash_keys, B * APSE_HASH_SLOTS * sizeof(unsigned long long)));
@@ -1251,7 +1250,7 @@ int apse_detect_alloc(apse_ctx *ctx)
 
 void apse_detect_free(apse_ctx *ctx)
 {
-    cudaFree(ctx->thresh); cudaFree(ctx->tmm_buf[0]); cudaFree(ctx->tmm_buf[1]); cudaFree(ctx->labels); cudaFree(ctx->points);
+    cudaFree(ctx->thresh); cudaFree(ctx->slot[0].tmm); cudaFree(ctx->slot[1].tmm); cudaFree(ctx->labels); cudaFree(ctx->points);
     cudaFree(ctx->hash_keys); cudaFree(ctx->hash_count); cudaFree(ctx->hash_offset); cudaFree(ctx->sorted_pts);
     cudaFree(ctx->sort_keys); cudaFree(ctx->lfps); cudaFree(ctx->errs); cudaFree(ctx->clusters); cudaFree(ctx->counters);
     cudaFree(ctx->quads); cudaFree(ctx->quad_order); cudaFree(ctx->quad_keys);
@@ -1272,7 +1271,7 @@ static int chain_grid(const apse_ctx *ctx)
 
 // runs K2..K5 for `batch` gray frames; leaves quads / counters in the context scratch
 int apse_apriltag_quads(apse_ctx *ctx, const uint8_t *gray, int w, int h, int batch, const DeviceParams &dp, cudaStream_t st,
-                        bool have_tile_minmax, bool flat_labels)
+                        const TileSlot *tiles, uint16_t *tmm_scratch, bool flat_labels)
 {
     if (w > ctx->max_w || h > ctx->max_h || batch > ctx->max_batch || batch > 64)
         CTX_FAIL(ctx, APSE_ERR_INVALID_ARG, "detect: frame %dx%d x%d exceeds the context capacity %dx%d x%d (64 max)", w, h,
@@ -1300,19 +1299,20 @@ int apse_apriltag_quads(apse_ctx *ctx, const uint8_t *gray, int w, int h, int ba
     int *acount = ex->work_counter + 2 + cur;
     {
         dim3 block(32, 8), grid(div_up(tw, 32), div_up(th, 8), batch);
-        if (!have_tile_minmax)
-            KLAUNCH(ctx, KID_TILE_MINMAX, st, k_tile_minmax<<<grid, block, 0, st>>>(gray, w, h, tw, th, ctx->tmm));
-        if (have_tile_minmax && ctx->sparse_active && ctx->sparse_elist && tw * 4 == w && th * 4 == h) {
-            KLAUNCH(ctx, KID_THRESHOLD, st, k_threshold_scan_list<<<chain_grid(ctx), 256, 0, st>>>(tw, th, ctx->tmm, ctx->sparse_elist, ctx->sparse_ecount,
+        uint16_t *tmm = tiles ? tiles->tmm : tmm_scratch;
+        if (!tiles)
+            KLAUNCH(ctx, KID_TILE_MINMAX, st, k_tile_minmax<<<grid, block, 0, st>>>(gray, w, h, tw, th, tmm));
+        if (tiles && tiles->bgr && tw * 4 == w && th * 4 == h) {   // sparse batch: scan only its exact tiles
+            KLAUNCH(ctx, KID_THRESHOLD, st, k_threshold_scan_list<<<chain_grid(ctx), 256, 0, st>>>(tw, th, tmm, tiles->elist, tiles->ecount,
                                                                                              dp.min_white_black_diff, ex->alist[cur], ex->alist_thr[cur], acount,
                                                                                              ex->acap, ex->tile_active, ctw, cth));
         } else {
             dim3 tgrid(div_up(div_up(tw, THR_TPT), 128), th, batch);
-            KLAUNCH(ctx, KID_THRESHOLD, st, k_threshold_scan<<<tgrid, 128, 0, st>>>(w, h, tw, th, ctx->tmm, dp.min_white_black_diff, ex->alist[cur],
+            KLAUNCH(ctx, KID_THRESHOLD, st, k_threshold_scan<<<tgrid, 128, 0, st>>>(w, h, tw, th, tmm, dp.min_white_black_diff, ex->alist[cur],
                                                                                    ex->alist_thr[cur], acount, ex->acap, ex->tile_active, ctw, cth));
         }
         if (tw * 4 != w || th * 4 != h) {
-            KLAUNCH(ctx, KID_THRESHOLD, st, k_threshold_edges<<<dim3(64, 1, batch), 256, 0, st>>>(gray, w, h, tw, th, ctx->tmm, ctx->thresh,
+            KLAUNCH(ctx, KID_THRESHOLD, st, k_threshold_edges<<<dim3(64, 1, batch), 256, 0, st>>>(gray, w, h, tw, th, tmm, ctx->thresh,
                                                                                      ex->tile_active, ctw, cth, ex->alist[cur], ex->alist_thr[cur],
                                                                                      acount, ex->acap));
         }

@@ -879,11 +879,10 @@ void apse_sparse_free(apse_ctx *ctx)
 {
     cudaFree(ctx->btable);
     if (ctx->aux_stream) { cudaStreamDestroy(ctx->aux_stream); cudaEventDestroy(ctx->aux_ev[0]); cudaEventDestroy(ctx->aux_ev[1]); }
-    for (int k = 0; k < 2; k++) { cudaFree(ctx->tbounds[k]); cudaFree(ctx->eflag[k]); cudaFree(ctx->elist[k]); cudaFree(ctx->ecount[k]); }
+    for (TileSlot &s : ctx->slot) { cudaFree(s.tbounds); cudaFree(s.eflag); cudaFree(s.elist); cudaFree(s.ecount); }
 }
 
-int apse_preprocess_sparse(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gray, uint16_t *tmm, int slot, int batch, int min_wb_diff,
-                           cudaStream_t st)
+int apse_preprocess_sparse(apse_ctx *ctx, TileSlot &slot, const uint8_t *bgr, uint8_t *gray, int batch, int min_wb_diff, cudaStream_t st)
 {
     const int w = ctx->w, h = ctx->h;
     PFN_tmapEncodeTiled enc = get_tmap_encoder();
@@ -902,11 +901,11 @@ int apse_preprocess_sparse(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gray, uin
     }
     const int tw = w / 4, th = h / 4;
     const size_t ntiles = (size_t)ctx->max_batch * (ctx->max_w / 4) * (ctx->max_h / 4);
-    if (!ctx->tbounds[slot]) {
-        CUDA_TRY(ctx, cudaMalloc((void **)&ctx->tbounds[slot], ntiles * sizeof(uint16_t)));
-        CUDA_TRY(ctx, cudaMalloc((void **)&ctx->eflag[slot], ntiles));
-        CUDA_TRY(ctx, cudaMalloc((void **)&ctx->elist[slot], ntiles * sizeof(uint32_t)));
-        CUDA_TRY(ctx, cudaMalloc((void **)&ctx->ecount[slot], sizeof(int)));
+    if (!slot.tbounds) {
+        CUDA_TRY(ctx, cudaMalloc((void **)&slot.tbounds, ntiles * sizeof(uint16_t)));
+        CUDA_TRY(ctx, cudaMalloc((void **)&slot.eflag, ntiles));
+        CUDA_TRY(ctx, cudaMalloc((void **)&slot.elist, ntiles * sizeof(uint32_t)));
+        CUDA_TRY(ctx, cudaMalloc((void **)&slot.ecount, sizeof(int)));
     }
     // 4K bounds pass: 40 registers per thread (leaves 15 K registers per SM to co-resident chain CTAs; 48 has no spill) and a
     // staging ring of 3
@@ -918,8 +917,8 @@ int apse_preprocess_sparse(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gray, uin
     }
     const int nz = div_up(batch, 20), fpb = div_up(batch, nz);
     dim3 grid(div_up(w, P2_TW), div_up(h, P2_TH), nz);
-    CUDA_TRY(ctx, cudaMemsetAsync(ctx->ecount[slot], 0, sizeof(int), st));
-#define K1B_ARGS tmap, bgr, nullptr, nullptr, ctx->tbounds[slot], ctx->mapx, ctx->mapy, ctx->btable, w, h, batch, fpb
+    CUDA_TRY(ctx, cudaMemsetAsync(slot.ecount, 0, sizeof(int), st));
+#define K1B_ARGS tmap, bgr, nullptr, nullptr, slot.tbounds, ctx->mapx, ctx->mapy, ctx->btable, w, h, batch, fpb
     if (w == 3840 && h % P2_TH == 0)
         KLAUNCH(ctx, KID_PREPROCESS, st, k_preprocess_tma<false, 40, 3840, true, 1, 3><<<grid, P2_CTA_THREADS, P2_SMEM_BYTES_N(1, 3), st>>>(K1B_ARGS));
     else
@@ -939,9 +938,9 @@ int apse_preprocess_sparse(apse_ctx *ctx, const uint8_t *bgr, uint8_t *gray, uin
     CUDA_TRY(ctx, cudaEventRecord(ctx->aux_ev[0], st));
     CUDA_TRY(ctx, cudaStreamWaitEvent(sx, ctx->aux_ev[0], 0));
     KLAUNCH(ctx, KID_SPARSE_FLAGS, sx, k_sparse_flags<<<dim3(div_up(tw / 8, 128), div_up(th, SFL_ROWS), batch), 128, 0, sx>>>(
-                ctx->tbounds[slot], tw, th, min_wb_diff, tmm, ctx->eflag[slot], ctx->elist[slot], ctx->ecount[slot]));
-    KLAUNCH(ctx, KID_SPARSE_EXACT, sx, k_sparse_exact<<<ctx->sm_count * 6, 256, 0, sx>>>(bgr, ctx->mapx, ctx->mapy, ctx->tables2, w, h, ctx->elist[slot],
-                                                                                      ctx->ecount[slot], gray, tmm));
+                slot.tbounds, tw, th, min_wb_diff, slot.tmm, slot.eflag, slot.elist, slot.ecount));
+    KLAUNCH(ctx, KID_SPARSE_EXACT, sx, k_sparse_exact<<<ctx->sm_count * 6, 256, 0, sx>>>(bgr, ctx->mapx, ctx->mapy, ctx->tables2, w, h, slot.elist,
+                                                                                      slot.ecount, gray, slot.tmm));
     CUDA_TRY(ctx, cudaEventRecord(ctx->aux_ev[1], sx));
     CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->aux_ev[1], 0));
     return APSE_OK;
